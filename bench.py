@@ -7,12 +7,14 @@ One "step" = MXTensor.to_mx followed by MXTensor.to_dtype(bfloat16) for each of 
 types (10 kernel launches).  Metric: algorithmic GB/s = (2 + code + 1/32 bytes per element, once
 for quantize and once for dequantize) / device time.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU): the tensors are independent, every rank runs the
 same sweep on its own GPU (weak scaling, no data-path collective); time = max over ranks.
 `--impl reference` times the CPU oracle (oracle/, the restatement of the reference's own CPU
 path -- the Python reference itself cannot travel to the GPU box) with all host threads.
+`--dump-outputs DIR` writes a fixed sample of what the last timed step computed (see dump_outputs),
+so that two builds can be compared output for output on identical seeded inputs.
 """
 from __future__ import annotations
 
@@ -484,6 +486,23 @@ def tp70b_extras(world, rank):
 
 
 # ---------------------------------------------------------------------------------------------------
+DUMP_ROWS = 64  # 64 of the 16384 rows: ~39 MB of float32 over the five element types (codes, scales, dequantized values)
+
+
+def dump_outputs(outs, directory: str):
+    """Write what the caller of the timed path received in one step -- per element type the MXTensor's codes (`_data`) and E8M0
+    scales (`_scale_e8m0`) and the dequantized bf16 tensor -- restricted to the same DUMP_ROWS rows, picked with a fixed seed, as
+    float32 `<elem>_{codes,scales,dequantized}.npy` (every value is exact in float32: byte codes, scale bytes, bf16)."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    rows = torch.randperm(ROWS, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    for elem, (m, y) in zip(ELEMS, outs):
+        idx = rows.to(y.device)
+        for name, t in (("codes", m._data), ("scales", m._scale_e8m0), ("dequantized", y)):
+            np.save(os.path.join(directory, f"{elem}_{name}.npy"), t[idx].float().cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torchmx_b200  # noqa: F401  registers the ops; raises if libmxq.so is missing
@@ -519,6 +538,7 @@ def run_b200(args):
 
     def step(i, ev=None):
         x = xs[i % 3]
+        outs = []
         for j, et in enumerate(etypes):
             if ev is not None:
                 ev[j][0].record()
@@ -528,10 +548,13 @@ def run_b200(args):
             y = m.to_dtype(torch.bfloat16)
             if ev is not None:
                 ev[j][2].record()
-        return y
+            outs.append((m, y))
+        return outs
 
+    # Warm-up keeps each step's results alive the way the timed loop does, so the caching allocator already holds every block
+    # the timed loop asks for.
     for i in range(args.warmup):
-        step(i)
+        outs = step(i)
     # per-launch events (on the launching = current stream) for the roofline of the dominant kernel
     evs = [[[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in ELEMS] for _ in range(args.steps)]
     t_start, t_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -544,10 +567,13 @@ def run_b200(args):
     torch.cuda._sleep(20_000_000)
     t_start.record()
     for i in range(args.steps):
-        step(i, evs[i])
+        outs = step(i, evs[i])
     t_end.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(outs, args.dump_outputs)
+    del outs
     elapsed_ms = t_start.elapsed_time(t_end)
     if dist is not None:
         t = torch.tensor([elapsed_ms], device=dev)
@@ -736,7 +762,11 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="profiling runs only: skip the cpu_baseline leg")
     ap.add_argument("--skip-gemm", action="store_true", help="skip the secondary MX matmul numbers (rank 0, after the timed sweep)")
     ap.add_argument("--skip-llama", action="store_true", help="skip the MX-Llama extras (8B through the public API at N = 1, 70B tensor-parallel at every N)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed row sample of the last step's codes, scales and "
+                                                          "dequantized tensors of every element type to DIR/<name>.npy (float32, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
