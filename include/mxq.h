@@ -383,6 +383,43 @@ typedef struct {
 } mxq_transposed_quantize_args_t;
 MXQ_API int mxq_quantize_transposed(const mxq_transposed_quantize_args_t *args, int device, void *stream);
 
+/*
+ * rotary embedding + append to an MX-quantized static KV cache + quantization of Q, as ONE launch  <->  the MX attention block's
+ *     q, k = apply_rotary_pos_emb(q, k, cos, sin);  keys, values = StaticCache.update(k, v)       (bf16 cache of capacity C)
+ *     Q = to_mx(q);  K = to_mx(keys);  Vt = to_mx(transpose(values, -2, -1))                      (mxq_rope + mxq_quantize + mxq_quantize_transposed)
+ * where only the new tokens' blocks are computed: K is blocked along head_dim, so a key row's codes depend on that row alone;
+ * V is blocked along 32 consecutive positions, and every V block that [L, L + tokens) touches is re-derived from v_open (the bf16
+ * positions of the block holding L below L), the new values, and zeros at and past L + tokens -- the same bytes the whole-cache
+ * quantization of a zero-initialised bf16 cache gives.  Rotary arithmetic = mxq_rope's, block arithmetic = mxq_quantize's.
+ *   q / k / v : bf16, element (b, t, h, d) at  base + b*batch_stride + t*tok_stride + h*head_dim + d  (projection outputs, possibly
+ *               column slices of one stacked q/k/v output, read in place); strides multiples of 8 elements, 16-byte aligned bases
+ *   cos/sin   : bf16 [batch | 1, tokens, head_dim] (cs_batch_stride 0 broadcasts)
+ *   q_elem, k_elem, v_elem : any floating-point mxq_elem_t (MXQ_ELEM_INT8 -> MXQ_ERR_INVALID); flags: MXQ_FLAG_HW_EXACT
+ * Storage, one byte per element in the form mxq_flash_attention reads: e4m3 / e5m2 codes as they are, fp6 / fp4 codes re-encoded
+ * exactly as E4M3 (what mxq_transcode_to_e4m3 produces); 32-byte aligned bases:
+ *   q_codes  : [batch, q_heads, tokens, 128], q_scales [batch, q_heads, tokens, 4]          (written)
+ *   k_codes  : [batch, kv_heads, C, 128],     k_scales [batch, kv_heads, C, 4]              (rows L .. L + tokens - 1 written)
+ *   vt_codes : [batch, kv_heads, 128, C],     vt_scales [batch, kv_heads, 128, C / 32]      (blocks touched by [L, L + tokens))
+ *   v_open   : bf16 [batch, kv_heads, 32, 128]: read as the block holding L, left holding the block holding L + tokens
+ *   position : DEVICE pointer to the int64 write position L (read, not advanced: a captured step replays as the caller advances it)
+ * Positions at or past C are dropped.  head_dim must be 128 (MXQ_ERR_UNSUPPORTED_SHAPE otherwise, and for misaligned operands);
+ * C % 32 != 0, tokens > C or a NULL pointer is MXQ_ERR_INVALID.
+ */
+typedef struct {
+    const void *q; int64_t q_tok_stride, q_batch_stride; int q_heads;
+    const void *k; int64_t k_tok_stride, k_batch_stride;
+    const void *v; int64_t v_tok_stride, v_batch_stride; int kv_heads;
+    const void *cos; const void *sin; int64_t cs_tok_stride, cs_batch_stride;
+    int64_t batch, tokens; int head_dim;
+    int q_elem, k_elem, v_elem /* mxq_elem_t */; unsigned flags /* MXQ_FLAG_HW_EXACT */;
+    void *q_codes; uint8_t *q_scales;
+    void *k_codes; uint8_t *k_scales;
+    void *vt_codes; uint8_t *vt_scales;
+    void *v_open;
+    int64_t capacity; const int64_t *position;
+} mxq_rope_quantize_kv_args_t;
+MXQ_API int mxq_rope_quantize_kv(const mxq_rope_quantize_kv_args_t *args, int device, void *stream);
+
 #define MXQ_OK 0
 #define MXQ_ERR_INVALID 1
 #define MXQ_ERR_UNSUPPORTED_SHAPE 2

@@ -6,6 +6,9 @@ Timed with CUDA events; "graph" lines replay a captured CUDA graph of the same f
 number), "eager" lines include the Python dispatch of the reference-style module stack.
 
     python tools/llama_bench.py --model 8b [--layers N] [--prefill 2048] [--batch 32] [--steps 64]
+
+--llm-api --mx-attention --mx-kv-cache keeps the KV cache as MX codes (torchmx_b200.kv_cache.MXStaticCache) instead of HF's bf16
+StaticCache; `kv_cache_bytes` is the resident size of the decode cache either way.
 """
 from __future__ import annotations
 
@@ -105,6 +108,12 @@ def set_len(cache, n: int) -> None:
             layer.cumulative_length.fill_(n)
 
 
+def kv_cache_bytes(cache) -> int:
+    """bytes the cache's layers hold: bf16 keys / values, or MX codes, scales and open value blocks"""
+    names = ("k_codes", "k_scales", "vt_codes", "vt_scales", "v_open", "keys", "values")
+    return sum(t.numel() * t.element_size() for layer in cache.layers for t in (getattr(layer, n, None) for n in names) if isinstance(t, torch.Tensor))
+
+
 def capture(fn):
     s = torch.cuda.Stream()
     s.wait_stream(torch.cuda.current_stream())
@@ -123,9 +132,14 @@ def capture(fn):
 def run(args) -> dict:
     from transformers.cache_utils import StaticCache
 
+    if args.mx_kv_cache:
+        if not (args.llm_api and args.mx_attention):
+            raise SystemExit("--mx-kv-cache needs --llm-api --mx-attention (the cache holds the MX attention operands)")
+        from torchmx_b200.kv_cache import MXStaticCache as StaticCache  # noqa: F811
     model, cfg, info = build(args.model, args.layers, args.wdtype, args.adtype, quantize=not args.no_quant, llm_api=args.llm_api, mx_attention=args.mx_attention,
                              fuse_norm=getattr(args, "fuse_norm", None))
-    res = {"api": "none (bf16 HF)" if args.no_quant else (("quantize_llm_ + MX attention" if args.mx_attention else "quantize_llm_") if args.llm_api else "quantize_linear_"), "model": args.model, "layers": cfg.num_hidden_layers, "weights": args.wdtype, "activations": args.adtype, **info}
+    res = {"api": "none (bf16 HF)" if args.no_quant else (("quantize_llm_ + MX attention" if args.mx_attention else "quantize_llm_") if args.llm_api else "quantize_linear_"),
+           "kv_cache": "MXStaticCache" if args.mx_kv_cache else "StaticCache", "model": args.model, "layers": cfg.num_hidden_layers, "weights": args.wdtype, "activations": args.adtype, **info}
     dev = "cuda"
 
     # ---- prefill: one prompt of `prefill` tokens, fresh static cache each run -------------------------------
@@ -134,7 +148,7 @@ def run(args) -> dict:
     cache = StaticCache(config=cfg, max_cache_len=-(-(P + 8) // 128) * 128 if args.mx_attention else P + 8)  # MX attention contractions need a multiple of 128
 
     def prefill():
-        set_len(cache, 0)
+        set_len(cache, 0)  # (also for the MX cache: codes left past the prompt are masked, and crop would synchronise inside a capture)
         return model(input_ids=ids, past_key_values=cache, use_cache=True).logits
 
     ms = time_fn(prefill, args.prefill_iters)
@@ -165,7 +179,10 @@ def run(args) -> dict:
         return logits
 
     def decode_run(step_fn):
-        set_len(cache, ctx)
+        if args.mx_kv_cache:
+            cache.crop(ctx)
+        else:
+            set_len(cache, ctx)
         for _ in range(steps):
             step_fn()
 
@@ -174,13 +191,17 @@ def run(args) -> dict:
     res["decode_eager_tok_s"] = B / ms * 1e3
     if not args.no_graph:
         try:
-            set_len(cache, ctx)
+            if args.mx_kv_cache:
+                cache.crop(ctx)
+            else:
+                set_len(cache, ctx)
             g, _ = capture(decode_step)
             ms = time_fn(lambda: decode_run(g.replay), 2, warmup=1) / steps
             res["decode_graph_ms_per_step"] = ms
             res["decode_graph_tok_s"] = B / ms * 1e3
         except Exception as e:  # noqa: BLE001
             res["decode_graph_error"] = f"{type(e).__name__}: {str(e)[:300]}"
+    res["kv_cache_bytes"] = kv_cache_bytes(cache)
     codes_bytes = info["weight_elements"] * ((0.5 if args.wdtype == "float4_e2m1" else 1) + 1 / 32)
     res["decode_weight_stream_floor_ms"] = codes_bytes / 6.5e12 * 1e3
     from torchmx_b200 import mx_gemm
@@ -195,7 +216,7 @@ def run(args) -> dict:
 def run_cfg(**kw) -> dict:
     """`run` with keyword arguments (bench.py calls this in-process): defaults = the command line's"""
     base = dict(model="8b", layers=None, prefill=2048, prefill_iters=5, batch=32, ctx=128, steps=64, wdtype="float6_e3m2", adtype="float8_e4m3",
-                no_graph=False, llm_api=False, mx_attention=False, no_quant=False, fuse_norm=None)
+                no_graph=False, llm_api=False, mx_attention=False, no_quant=False, fuse_norm=None, mx_kv_cache=False)
     base.update(kw)
     return run(argparse.Namespace(**base))
 
@@ -214,6 +235,7 @@ if __name__ == "__main__":
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--llm-api", action="store_true", help="quantize_llm_ (MX attention / MLP blocks) instead of quantize_linear_")
     ap.add_argument("--mx-attention", action="store_true", help="with --llm-api: quantize Q, K, V and the attention probabilities (MX bmm + fused softmax)")
+    ap.add_argument("--mx-kv-cache", action="store_true", help="with --llm-api --mx-attention: the KV cache held as MX codes (MXStaticCache)")
     ap.add_argument("--no-quant", action="store_true", help="plain bf16 HF model (context line, not the product)")
     ap.add_argument("--pack", action="store_true", help="pack_linear_: weights held only as packed tensor-core operands")
     a = ap.parse_args()

@@ -14,11 +14,12 @@ HP_BF16, HP_F32 = 0, 1
 FLAG_HW_EXACT = 1
 FLAG_OPERAND_LAYOUT = 2
 GEMM_B_STATIC, GEMM_WIDE_TILES, GEMM_NO_PDL, GEMM_NO_MXF4 = 1, 2, 4, 8
-ABI_VERSION = 3
+ABI_VERSION = 4
 MAX_DIMS = 6
 
 EXPORTS = ("mxq_quantize", "mxq_dequantize", "mxq_dequantize_strided", "mxq_gemm", "mxq_gemm_dequant", "mxq_gemm_bf16", "mxq_transcode_to_e4m3", "mxq_pack_operand", "mxq_unpack_operand",
-           "mxq_softmax_quantize", "mxq_flash_attention", "mxq_silu_mul_quantize", "mxq_rmsnorm", "mxq_rope", "mxq_quantize_heads", "mxq_quantize_transposed", "mxq_last_error", "mxq_version", "mxq_arch")
+           "mxq_softmax_quantize", "mxq_flash_attention", "mxq_silu_mul_quantize", "mxq_rmsnorm", "mxq_rope", "mxq_quantize_heads", "mxq_quantize_transposed", "mxq_rope_quantize_kv",
+           "mxq_last_error", "mxq_version", "mxq_arch")
 
 
 class GemmArgs(ctypes.Structure):
@@ -118,6 +119,22 @@ class TransposedQuantArgs(ctypes.Structure):
     ]
 
 
+class RopeQuantizeKVArgs(ctypes.Structure):
+    _fields_ = [
+        ("q", ctypes.c_void_p), ("q_tok_stride", ctypes.c_int64), ("q_batch_stride", ctypes.c_int64), ("q_heads", ctypes.c_int),
+        ("k", ctypes.c_void_p), ("k_tok_stride", ctypes.c_int64), ("k_batch_stride", ctypes.c_int64),
+        ("v", ctypes.c_void_p), ("v_tok_stride", ctypes.c_int64), ("v_batch_stride", ctypes.c_int64), ("kv_heads", ctypes.c_int),
+        ("cos", ctypes.c_void_p), ("sin", ctypes.c_void_p), ("cs_tok_stride", ctypes.c_int64), ("cs_batch_stride", ctypes.c_int64),
+        ("batch", ctypes.c_int64), ("tokens", ctypes.c_int64), ("head_dim", ctypes.c_int),
+        ("q_elem", ctypes.c_int), ("k_elem", ctypes.c_int), ("v_elem", ctypes.c_int), ("flags", ctypes.c_uint),
+        ("q_codes", ctypes.c_void_p), ("q_scales", ctypes.c_void_p),
+        ("k_codes", ctypes.c_void_p), ("k_scales", ctypes.c_void_p),
+        ("vt_codes", ctypes.c_void_p), ("vt_scales", ctypes.c_void_p),
+        ("v_open", ctypes.c_void_p),
+        ("capacity", ctypes.c_int64), ("position", ctypes.c_void_p),
+    ]
+
+
 _lib = None
 _lock = threading.Lock()
 
@@ -172,6 +189,8 @@ def lib() -> ctypes.CDLL:
         L.mxq_rope.argtypes = [ctypes.POINTER(RopeArgs), i32, vp]
         L.mxq_quantize_transposed.restype = i32
         L.mxq_quantize_transposed.argtypes = [ctypes.POINTER(TransposedQuantArgs), i32, vp]
+        L.mxq_rope_quantize_kv.restype = i32
+        L.mxq_rope_quantize_kv.argtypes = [ctypes.POINTER(RopeQuantizeKVArgs), i32, vp]
         if L.mxq_version() != ABI_VERSION:
             raise RuntimeError(f"torchmx_b200: libmxq.so has ABI v{L.mxq_version()}, this package needs v{ABI_VERSION}: rebuild with `python -m torchmx_b200.build --force`")
         if L.mxq_arch() != 1000:

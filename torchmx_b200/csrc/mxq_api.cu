@@ -26,6 +26,7 @@ int launch_rmsnorm(const mxq_rmsnorm_args_t*, cudaStream_t, char*, size_t);
 int launch_rope(const mxq_rope_args_t*, int, cudaStream_t, char*, size_t);
 int launch_heads_quantize(const void*, int64_t, int64_t, int64_t, int64_t, int, unsigned, void*, uint8_t*, cudaStream_t, char*, size_t);
 int launch_transposed_quantize(const mxq_transposed_quantize_args_t*, cudaStream_t, char*, size_t);
+int launch_rope_quantize_kv(const mxq_rope_quantize_kv_args_t*, cudaStream_t, char*, size_t);
 }  // namespace mxq
 
 namespace {
@@ -87,7 +88,7 @@ int waves_override() { static int v = env_int("MXQ_WAVES"); return v > 0 ? v : 0
 extern "C" {
 
 const char* mxq_last_error(void) { return g_err; }
-int mxq_version(void) { return 3; }
+int mxq_version(void) { return 4; }
 int mxq_arch(void) { return 1000; }
 
 int mxq_quantize(const void* src, int src_dtype, int64_t n_blocks, int block_size, int elem, unsigned flags, void* codes, uint8_t* scales,
@@ -320,6 +321,26 @@ int mxq_softmax_quantize(const mxq_softmax_args_t* a, int device, void* stream) 
     char msg[400] = "";
     const int rc = mxq::launch_softmax_quantize(a, (cudaStream_t)stream, msg, sizeof(msg));
     return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_softmax_quantize: %s", msg);
+}
+
+int mxq_rope_quantize_kv(const mxq_rope_quantize_kv_args_t* a, int device, void* stream) {
+    if (!a) return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: null args");
+    for (int e : {a->q_elem, a->k_elem, a->v_elem})
+        if (!valid_elem(e) || e == MXQ_ELEM_INT8) return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: element type %d has no one-byte attention operand", e);
+    if (a->batch < 0 || a->tokens < 0 || a->q_heads < 0 || a->kv_heads < 0) return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: negative extent");
+    if (a->capacity <= 0 || a->capacity % 32 || a->tokens > a->capacity)
+        return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: capacity %lld must be a positive multiple of 32 and hold %lld tokens", (long long)a->capacity, (long long)a->tokens);
+    if (a->batch == 0 || a->tokens == 0) return MXQ_OK;
+    if (a->q_heads == 0 || a->kv_heads == 0) return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: no heads");
+    if (!a->q || !a->k || !a->v || !a->cos || !a->sin || !a->q_codes || !a->q_scales || !a->k_codes || !a->k_scales || !a->vt_codes || !a->vt_scales ||
+        !a->v_open || !a->position)
+        return fail(MXQ_ERR_INVALID, "mxq_rope_quantize_kv: null pointer");
+    if (a->head_dim != 128) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_rope_quantize_kv: needs head_dim == 128 (got %d)", a->head_dim);
+    DeviceScope scope(device);
+    if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_rope_quantize_kv: selecting device");
+    char msg[400] = "";
+    const int rc = mxq::launch_rope_quantize_kv(a, (cudaStream_t)stream, msg, sizeof(msg));
+    return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_rope_quantize_kv: %s", msg);
 }
 
 }  // extern "C"

@@ -13,16 +13,13 @@
 #include <cstdio>
 
 #include "mxq_quant_core.cuh"
+#include "mxq_rope_core.cuh"
 
 namespace mxq {
 namespace glue {
 
 constexpr int kNormThreads = 256;
 constexpr int MAX_CHUNKS = 4;  // 16-element chunks per thread: hidden <= 16 * 256 * 4 = 16384
-
-__device__ __forceinline__ float bf16lo(uint32_t w) { return __uint_as_float(w << 16); }
-__device__ __forceinline__ float bf16hi(uint32_t w) { return __uint_as_float(w & 0xFFFF0000u); }
-__device__ __forceinline__ float round_bf16(float f) { return __uint_as_float(pack_bf16x2(f, 0.0f) << 16); }
 
 struct NormParams {
     const uint16_t* x; int64_t ldx;
@@ -168,13 +165,8 @@ __global__ void __launch_bounds__(256) rope_kernel(const RopeParams p) {
         uint32_t o1[4], o2[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-            // q_embed = (q * cos) + (rotate_half(q) * sin), rotate_half = cat(-x2, x1): each product and the sum are bf16 tensors
-            const float lo1 = round_bf16(bf16lo(a1[j]) * bf16lo(k1[j])) + round_bf16(-bf16lo(a2[j]) * bf16lo(z1[j]));
-            const float hi1 = round_bf16(bf16hi(a1[j]) * bf16hi(k1[j])) + round_bf16(-bf16hi(a2[j]) * bf16hi(z1[j]));
-            const float lo2 = round_bf16(bf16lo(a2[j]) * bf16lo(k2[j])) + round_bf16(bf16lo(a1[j]) * bf16lo(z2[j]));
-            const float hi2 = round_bf16(bf16hi(a2[j]) * bf16hi(k2[j])) + round_bf16(bf16hi(a1[j]) * bf16hi(z2[j]));
-            o1[j] = pack_bf16x2(lo1, hi1);
-            o2[j] = pack_bf16x2(lo2, hi2);
+            o1[j] = rope_first_half(a1[j], a2[j], k1[j], z1[j]);
+            o2[j] = rope_second_half(a2[j], a1[j], k2[j], z2[j]);
         }
         *reinterpret_cast<uint4*>(dst) = make_uint4(o1[0], o1[1], o1[2], o1[3]);
         *reinterpret_cast<uint4*>(dst + hd2) = make_uint4(o2[0], o2[1], o2[2], o2[3]);

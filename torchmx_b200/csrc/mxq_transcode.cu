@@ -2,17 +2,9 @@
 // byte with the even element in the high nibble) as E4M3 bytes.  Every e3m2 / e2m3 / e2m1 value is
 // an e4m3 value, so the block-scaled tensor-core path can consume all FP element types as
 // kind::mxf8f6f4 E4M3 operands without touching the reference's persisted storage layout.
-#include "mxq_common.cuh"
+#include "mxq_transcode_core.cuh"
 
 namespace mxq {
-
-template <int ELEM>
-__device__ __forceinline__ uint32_t to_e4m3_pair(uint32_t h2) {
-    // f16x2 -> two e4m3 bytes (exact: the value set is a subset of e4m3)
-    uint16_t r;
-    asm("cvt.rn.satfinite.e4m3x2.f16x2 %0, %1;" : "=h"(r) : "r"(h2));
-    return r;
-}
 
 template <int ELEM>
 __global__ void __launch_bounds__(256) transcode_kernel(const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int64_t n_in_bytes) {
@@ -24,30 +16,14 @@ __global__ void __launch_bounds__(256) transcode_kernel(const uint8_t* __restric
         const uint32_t w[4] = {v.x, v.y, v.z, v.w};
         if constexpr (ELEM == MXQ_ELEM_E2M1) {
             uint32_t o[8];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-#pragma unroll
-                for (int k = 0; k < 2; ++k) {
-                    const uint32_t b0 = (w[j] >> (16 * k)) & 0xFF, b1 = (w[j] >> (16 * k + 8)) & 0xFF;
-                    const uint32_t h0 = decode_e2m1_byte_f16x2(b0), h1 = decode_e2m1_byte_f16x2(b1);
-                    // high nibble (high half) is the earlier element -> swap halves
-                    const uint32_t p0 = to_e4m3_pair<ELEM>(__byte_perm(h0, 0, 0x1032));
-                    const uint32_t p1 = to_e4m3_pair<ELEM>(__byte_perm(h1, 0, 0x1032));
-                    o[2 * j + k] = p0 | (p1 << 16);
-                }
-            }
+            transcode_words_to_e4m3<ELEM, 4>(w, o);
             u32x8 r;
 #pragma unroll
             for (int k = 0; k < 8; ++k) r.v[k] = o[k];
             stg256_stream(out + i * 32, r);
         } else {
             uint32_t o[4];
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                const uint32_t p0 = to_e4m3_pair<ELEM>(decode_pair_f16x2<ELEM>(w[j] & 0xFFFF));
-                const uint32_t p1 = to_e4m3_pair<ELEM>(decode_pair_f16x2<ELEM>(w[j] >> 16));
-                o[j] = p0 | (p1 << 16);
-            }
+            transcode_words_to_e4m3<ELEM, 4>(w, o);
             stg128_stream(out + i * 16, make_uint4(o[0], o[1], o[2], o[3]));
         }
     }
@@ -55,12 +31,11 @@ __global__ void __launch_bounds__(256) transcode_kernel(const uint8_t* __restric
     for (int64_t b = n_vec * 16 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; b < n_in_bytes; b += stride) {
         const uint32_t c = in[b];
         if constexpr (ELEM == MXQ_ELEM_E2M1) {
-            const uint32_t h = decode_e2m1_byte_f16x2(c);
-            const uint32_t p = to_e4m3_pair<ELEM>(__byte_perm(h, 0, 0x1032));
+            const uint32_t p = e4m3_pair_from_fp4_byte(c);
             out[2 * b] = (uint8_t)p;
             out[2 * b + 1] = (uint8_t)(p >> 8);
         } else {
-            out[b] = (uint8_t)to_e4m3_pair<ELEM>(decode_pair_f16x2<ELEM>(c));
+            out[b] = (uint8_t)to_e4m3_pair(decode_pair_f16x2<ELEM>(c));
         }
     }
 }

@@ -7,6 +7,8 @@ linears of a Llama / Qwen2 decoder layer, each as ONE launch.
   (reference: torchmx/layers/mx_linear.py:63-66) -- the codes are bit-identical to `MXTensor.to_mx` of the bf16 norm output.
 * `rope(q, k, cos, sin)`: `apply_rotary_pos_emb` of transformers (reference call site: torchmx/layers/mx_llama_attention.py:171-187)
   with every bf16 rounding of the eager chain reproduced, reading the projection outputs in place.
+* `rope_quantize_kv(...)` (K5e, csrc/mxq_kv_cache.cu): rope, the append to an MX-quantized static KV cache and the quantization of
+  Q in one launch (the cache itself: torchmx_b200/kv_cache.py).
 
 Both return None when the operands do not qualify (the caller runs the module / the eager chain); there is no CPU path.
 """
@@ -22,7 +24,7 @@ from . import env_variables as env
 from .mlp_ops import _rows_view
 from .mx_tensor import MXTensor, _stream_ptr
 
-stats = {"rmsnorm": 0, "rmsnorm_to_mx": 0, "rope": 0, "quantize_heads": 0, "quantize_transposed": 0}
+stats = {"rmsnorm": 0, "rmsnorm_to_mx": 0, "rope": 0, "quantize_heads": 0, "quantize_transposed": 0, "rope_quantize_kv": 0}
 _ENABLED = os.environ.get("MXQ_FUSED_GLUE", "1") != "0"
 MAX_HIDDEN = 16384
 
@@ -200,3 +202,63 @@ def quantize_transposed(x: torch.Tensor, elem_dtype: dtypes.DType, block_size: i
     _C.check(rc, "mxq_quantize_transposed")
     stats["quantize_transposed"] += 1
     return MXTensor(scales, codes, elem_dtype, 32, torch.bfloat16)
+
+
+def byte_operand_dtype(elem_dtype: dtypes.DType) -> dtypes.DType:
+    """The element type whose one-byte codes hold `elem_dtype`'s values in the form K4b reads: e4m3 / e5m2 themselves, fp6 / fp4
+    as their exact E4M3 re-encoding (every e3m2 / e2m3 / e2m1 value is an e4m3 value)"""
+    return dtypes.float8_e5m2 if elem_dtype == dtypes.float8_e5m2 else dtypes.float8_e4m3
+
+
+def rope_quantize_kv(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor, position: torch.Tensor,
+                     k_codes: torch.Tensor, k_scales: torch.Tensor, vt_codes: torch.Tensor, vt_scales: torch.Tensor, v_open: torch.Tensor,
+                     elem_dtypes: Tuple[dtypes.DType, dtypes.DType, dtypes.DType]) -> Optional[MXTensor]:
+    """K5e: rotary embedding of q / k, the append of the rotated keys and of v to an MX-quantized static KV cache at the device
+    position `position` (int64, one element; read, not advanced), and the quantization of the rotated queries -- one launch.
+
+    q / k / v: [batch, heads, tokens, 128] transposed views of the projection outputs (as for `rope`); cos / sin: bf16
+    [batch | 1, tokens, 128].  The cache (uint8, contiguous, capacity C): k_codes [b, hk, C, 128], k_scales [b, hk, C, 4],
+    vt_codes [b, hk, 128, C], vt_scales [b, hk, 128, C / 32], v_open bf16 [b, hk, 32, 128].  `elem_dtypes`: the element types of
+    Q, K and V; codes are stored as `byte_operand_dtype` codes.  Returns Q as an MXTensor [b, hq, tokens, 128] of that storage
+    type, or None when the kernel does not apply."""
+    if not all(_plain_bf16(t, q.device) for t in (q, k, v, cos, sin)) or q.dim() != 4 or k.dim() != 4 or q.numel() == 0:
+        return None
+    if any(e == dtypes.int8 for e in elem_dtypes):
+        return None
+    b, hq, t, d = q.shape
+    hk = k.shape[1]
+    if d != 128 or k.shape != (b, hk, t, d) or v.shape != k.shape or cos.shape != sin.shape or cos.dim() != 3 or cos.shape[0] not in (1, b) \
+            or cos.shape[1] != t or cos.shape[2] != d or cos.stride() != sin.stride() or cos.stride(2) != 1:
+        return None
+    qv, kv, vv = _head_view(q, d), _head_view(k, d), _head_view(v, d)
+    if qv is None or kv is None or vv is None:
+        return None
+    C = k_codes.shape[2]
+    want = ((k_codes, (b, hk, C, d)), (k_scales, (b, hk, C, d // 32)), (vt_codes, (b, hk, d, C)), (vt_scales, (b, hk, d, C // 32)))
+    if any(x.dtype != torch.uint8 or x.device != q.device or tuple(x.shape) != shp or not x.is_contiguous() for x, shp in want):
+        return None
+    if v_open.dtype != torch.bfloat16 or v_open.shape != (b, hk, 32, d) or not v_open.is_contiguous() or v_open.device != q.device:
+        return None
+    if position.dtype != torch.int64 or position.numel() != 1 or position.device != q.device:
+        return None
+    a = _C.RopeQuantizeKVArgs()
+    a.q, a.q_batch_stride, a.q_tok_stride, a.q_heads = q.data_ptr(), qv[0], qv[1], hq
+    a.k, a.k_batch_stride, a.k_tok_stride = k.data_ptr(), kv[0], kv[1]
+    a.v, a.v_batch_stride, a.v_tok_stride, a.kv_heads = v.data_ptr(), vv[0], vv[1], hk
+    a.cos, a.sin = cos.data_ptr(), sin.data_ptr()
+    a.cs_tok_stride = cos.stride(1) if t > 1 else d
+    a.cs_batch_stride = cos.stride(0) if cos.shape[0] > 1 else 0
+    a.batch, a.tokens, a.head_dim = b, t, d
+    a.q_elem, a.k_elem, a.v_elem = (dtypes.ELEM_ID[e.name] for e in elem_dtypes)
+    a.flags = _C.FLAG_HW_EXACT if env.MX_EXACT_QUANTIZATION == "True" else 0  # (e5m2 has no hardware-exact variant: the kernel ignores it there)
+    q_codes = torch.empty((b, hq, t, d), dtype=torch.uint8, device=q.device)
+    q_scales = torch.empty((b, hq, t, d // 32), dtype=torch.uint8, device=q.device)
+    a.q_codes, a.q_scales = q_codes.data_ptr(), q_scales.data_ptr()
+    a.k_codes, a.k_scales, a.vt_codes, a.vt_scales = k_codes.data_ptr(), k_scales.data_ptr(), vt_codes.data_ptr(), vt_scales.data_ptr()
+    a.v_open, a.capacity, a.position = v_open.data_ptr(), C, position.data_ptr()
+    rc = _C.lib().mxq_rope_quantize_kv(a, q.device.index, _stream_ptr(q))
+    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+        return None
+    _C.check(rc, "mxq_rope_quantize_kv")
+    stats["rope_quantize_kv"] += 1
+    return MXTensor(q_scales, q_codes, byte_operand_dtype(elem_dtypes[0]), 32, torch.bfloat16)

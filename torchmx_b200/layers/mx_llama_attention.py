@@ -11,7 +11,10 @@ past_key_values, **kwargs) -> (attn_output, attn_weights)`), not the 4.44 intern
   extents are multiples of 128 (otherwise the dequantize path, like the reference), and everything between them is one
   kernel (`attention_ops.softmax_to_mx`, K4a) when the key/value length is a multiple of 32;
 * without it the module keeps the model's configured attention function (sdpa / flash / eager) on the rotated bf16 Q, K, V.
-The KV cache stays in high precision (reference :186-187).
+With HF's caches the KV cache stays in high precision (reference :186-187) and, with a full `QAttentionConfig`, the whole cache is
+quantized again at every forward.  With an `MXStaticCache` (torchmx_b200/kv_cache.py) and a full `QAttentionConfig` the cache holds
+the MX codes themselves: one launch (K5e) rotates, quantizes Q and appends only the new tokens' blocks, and the attention reads the
+cache in place -- the same codes, so the same logits as with a bf16 StaticCache.
 """
 from __future__ import annotations
 
@@ -23,6 +26,7 @@ from torch import nn
 
 from .. import attention_ops, glue_ops, mlp_ops, mx_gemm
 from ..config import QAttentionConfig, QLinearConfig
+from ..kv_cache import MXStaticCache
 from ..mx_tensor import MXTensor
 from .mx_linear import MXInferenceLinear
 
@@ -320,7 +324,6 @@ class _MXAttentionMixin:
         """reference :195-243; inputs [bs, heads, len, head_dim] after rotary / cache update -> [bs, q_len, heads, head_dim]"""
         qc = self.qconfig
         dtype = query_states.dtype
-        groups = self.num_key_value_groups
         q_mx = MXTensor.to_mx(query_states.contiguous(), qc.query_config.elem_dtype, qc.query_config.block_size)
         k_one = MXTensor.to_mx(key_states.contiguous(), qc.key_config.elem_dtype, qc.key_config.block_size)
         # V is quantized along the sequence axis (reference :205-212: transpose, quantize, transpose back): K5d reads the
@@ -329,6 +332,13 @@ class _MXAttentionMixin:
         vt_one = glue_ops.quantize_transposed(value_states, qc.value_config.elem_dtype, qc.value_config.block_size)
         if vt_one is None:
             vt_one = MXTensor.to_mx(value_states.transpose(2, 3).contiguous(), qc.value_config.elem_dtype, qc.value_config.block_size)
+        return self._mx_attend(q_mx, k_one, vt_one, attention_mask, scaling, dtype)
+
+    def _mx_attend(self, q_mx: MXTensor, k_one: MXTensor, vt_one: MXTensor, attention_mask, scaling: float, dtype: torch.dtype) -> torch.Tensor:
+        """the attention on MX operands: q_mx [bs, heads, q_len, head_dim], k_one [bs, kv_heads, kv_len, head_dim] and vt_one
+        [bs, kv_heads, head_dim, kv_len] (V quantized along the sequence) -> [bs, q_len, heads, head_dim]"""
+        qc = self.qconfig
+        groups = self.num_key_value_groups
         pc = qc.attention_weights_config
         q_len, kv_len = q_mx.shape[-2], k_one.shape[-2]
         mask, causal = None, False
@@ -383,6 +393,12 @@ class _MXAttentionMixin:
         key_states = k.view(hidden_shape).transpose(1, 2)
         value_states = v.view(hidden_shape).transpose(1, 2)
         cos, sin = position_embeddings
+        if isinstance(past_key_values, MXStaticCache) and self.qconfig.is_qkv_quantization_enabled:
+            # the cache holds MX codes: rotary, the quantization of Q and the append of the new tokens' K / V blocks are one launch
+            # (K5e), and the attention reads the whole cache in place
+            q_mx, k_mx, vt_mx = past_key_values.layers[self.layer_idx].mx_append(query_states, key_states, value_states, cos, sin, self.qconfig)
+            attn_output = self._mx_attend(q_mx, k_mx, vt_mx, attention_mask, self.scaling, query_states.dtype)
+            return self.o_proj(attn_output.reshape(*input_shape, -1).contiguous()), None
         rotated = glue_ops.rope(query_states, key_states, cos, sin)  # one launch, the eager chain's roundings (K5b)
         query_states, key_states = rotated if rotated is not None else mod_llama.apply_rotary_pos_emb(query_states, key_states, cos, sin)
         if past_key_values is not None:
