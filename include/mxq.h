@@ -281,9 +281,10 @@ MXQ_API int mxq_gemm_bf16(const void *a, int64_t lda, int64_t a_batch_stride, co
  *   out      : bf16, element (b, h, q, d) at out + b*out_batch_stride + h*out_head_stride + q*out_row_stride + d (so the caller
  *              picks [b, h, q, d] or the transposed [b, q, h, d] the reference produces next, :245)
  *   p_elem   : element type of P (any floating-point mxq_elem_t), flags: MXQ_FLAG_*
- * MXQ_ERR_UNSUPPORTED_SHAPE unless head_dim == 128, kv_len % 32 == 0, kv_len >= q_len, and the row is one whose block sums
- * mxq_softmax_quantize adds in an order this kernel reproduces (masked / causal: kv_len <= 8192; unmasked: kv_len <= 1024).
+ * MXQ_ERR_UNSUPPORTED_SHAPE unless head_dim == 128, kv_len % 32 == 0, q_len <= kv_len <= MXQ_FLASH_MAX_KV (masked or not).  Rows
+ * of any length add their block sums in mxq_softmax_quantize's order, including the lengths that entry point itself refuses.
  */
+#define MXQ_FLASH_MAX_KV 131072
 typedef struct {
     const void *q_codes; const uint8_t *q_scales; int q_format;
     const void *k_codes; const uint8_t *k_scales; int k_format;

@@ -21,6 +21,7 @@ stats = {"fused_softmax": 0, "unfused_softmax": 0, "flash_attention": 0}
 _ENABLED = os.environ.get("MXQ_FUSED_SOFTMAX", "1") != "0"
 _FLASH = os.environ.get("MXQ_FLASH_ATTENTION", "1") != "0"
 MAX_KV = 32768
+MAX_FLASH_KV = 131072  # the longest key axis K4b takes, masked or not (MXQ_FLASH_MAX_KV)
 
 
 def set_fused_softmax(on: bool) -> bool:
@@ -78,6 +79,22 @@ def set_flash_attention(on: bool) -> bool:
     return prev
 
 
+CHAIN_DECODE_MAX_CTAS = 16
+
+
+def chain_is_faster(batch: int, kv_heads: int, q_len: int, kv_len: int, masked: bool) -> bool:
+    """True for a decode step the K3 -> K4a -> K3 chain serves faster than K4b (same results either way: K4a takes the row).
+
+    K4b has no split over the key axis: a decode step is batch x kv_heads CTAs, each walking the whole key axis three times, and
+    costs about the same at 8 CTAs as at 256 (one wave).  The chain's cost grows with the batch instead.  On one B200 (1000 W),
+    Llama-3-8B heads (8 kv heads), unmasked, K4b against the chain at 2048 / 8192 / 32768 keys (profiles/r4_long_attention.json):
+    batch 1 (8 CTAs) 88 / 334 / 1322 us against 56 / 171 / 634; batch 2 (16 CTAs) 88 / 334 / 1330 against 87 / 315 / 1180;
+    batch 4 (32 CTAs) 92 / 347 / 1380 against 159 / 592 / 2293; batch 32 109 / 420 / 1632 against 1168 / 4517 / 18129.
+    Rows K4b took before it handled long key axes (up to 1024 keys unmasked, 8192 masked) stay with K4b."""
+    return (q_len == 1 and batch * kv_heads <= CHAIN_DECODE_MAX_CTAS and kv_len <= MAX_KV
+            and kv_len > (8192 if masked else 1024))
+
+
 def _byte_operand(t: MXTensor):
     """contiguous MXTensor blocked along its last dim -> (one-byte-per-element codes, MXQ_OPERAND_* format, scales) or None"""
     from . import mx_gemm
@@ -102,8 +119,7 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
     hk, kv_len = k_mx.shape[1], k_mx.shape[2]
     if d != 128 or k_mx.shape != (b, hk, kv_len, d) or vt_mx.shape != (b, hk, d, kv_len) or h % hk or kv_len % 32 or kv_len < q_len or q_len == 0:
         return None
-    masked = causal or mask is not None
-    if kv_len > (8192 if masked else 1024):  # (rows whose block sums K4a adds in an order K4b does not reproduce)
+    if kv_len > MAX_FLASH_KV:
         return None
     ops = [_byte_operand(t) for t in (q_mx, k_mx, vt_mx)]
     if any(o is None for o in ops):

@@ -28,8 +28,9 @@
 //   warp 18      scale-factor loader: Q / K / V E8M0 scales from their reference layout into the tcgen05.cp chunk layout
 // (At most 128 query rows per (batch, head) -- decode -- run a one-tile variant: eight softmax warps, two CTAs per SM; see Cfg.)
 // Causal attention without an explicit mask skips the key chunks a query tile's rows cannot see; with an explicit additive mask
-// pass A records the largest score of every (row, chunk) and passes B / C skip the chunks that are dead for a whole tile.
-// The key axis may be any multiple of 32 (a ragged last chunk is zero-filled by TMA and hidden).
+// pass A records the largest score of every (row, slot) and passes B / C skip the slots that are dead for a whole tile.  A slot
+// is 2^slot_shift consecutive chunks, as few as keep a row at 64 slots (one chunk per slot up to 8192 keys).
+// The key axis may be any multiple of 32 up to MXQ_FLASH_MAX_KV (a ragged last chunk is zero-filled by TMA and hidden).
 #include <cstring>
 
 #include "mxq_softmax_core.cuh"
@@ -76,8 +77,8 @@ struct SmemT {
     static constexpr int OFF_SFK = OFF_SFQ + TILES * 512;             // per stage: two 512-byte chunks (keys 0..63, 64..127)
     static constexpr int OFF_SFV = OFF_SFK + K_STAGES * 1024;
     static constexpr int OFF_SFP = OFF_SFV + V_STAGES * 512;
-    static constexpr int OFF_CMAX = OFF_SFP + TILES * 512;            // [wg][chunk <= 64][row] bf16: largest score of the chunk, from pass A
-    static constexpr int OFF_LIVE = OFF_CMAX + TILES * 64 * 128 * 2;  // [wg][2] words: chunks with a row that still counts after the row maximum is known
+    static constexpr int OFF_CMAX = OFF_SFP + TILES * 512;            // [wg][slot < 64][row] bf16: largest score of the slot's chunks, from pass A
+    static constexpr int OFF_LIVE = OFF_CMAX + TILES * 64 * 128 * 2;  // [wg][2] words: slots with a row that still counts after the row maximum is known
     static constexpr int OFF_XCH = OFF_LIVE + 16;                     // [wg][parity 2][sub 2][value 2][row 128] fp32: what a row's two threads exchange per chunk
     static constexpr int OFF_XMAX = OFF_XCH + TILES * 1024 * 4;       // [wg][sub][row] fp32: partial row maxima
     static constexpr int OFF_BAR = OFF_XMAX + TILES * 256 * 4;
@@ -98,6 +99,7 @@ struct Params {
     int batch, heads, kv_heads, q_len, kv_len;
     int causal, causal_offset, skip_hidden_chunks;
     int layout;  // sm::sum_layout of a row of kv_len / 32 blocks
+    int slot_shift;  // a live-chunk slot is 2^slot_shift chunks: the smallest that gives a row at most 64 slots
     float scaling;
     uint32_t idesc_qk, idesc_pv;
     uint32_t flags;
@@ -209,6 +211,9 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
     // everything anyway; it leaves the largest score of every (row, chunk) behind, and once a row's maximum is final a chunk whose
     // largest score lies more than 110 below it is +0 in every probability (sm::block_dead).  Chunks that are dead for all 128
     // rows of a warpgroup are skipped by passes B and C -- by the softmax threads, the tensor core and the loaders alike.
+    // The table and the live words hold one entry per SLOT of 2^slot_shift chunks (the slot's largest score; live if any of its
+    // chunks is).  A coarser slot only walks more chunks that turn out dead; a dead chunk adds +0 sums and +0 codes either way,
+    // so the slot width never changes a result.  Without a table every slot is live and only j < nv[wg] limits the walk.
     constexpr bool use_table = TABLE;  // (launched with TABLE == (mask != nullptr): the implied-causal path carries none of this)
     auto live_chunks = [&](uint64_t (&live)[2]) {  // (callers other than the softmax threads: waits for pass A of both warpgroups)
         live[0] = live[1] = 0;
@@ -219,10 +224,11 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 mbar_wait(&scan_done[wg], 0);
                 live[wg] = (uint64_t)live_words[2 * wg] | ((uint64_t)live_words[2 * wg + 1] << 32);
             } else {
-                live[wg] = nv[wg] >= 64 ? ~0ull : ((1ull << nv[wg]) - 1);
+                live[wg] = ~0ull;
             }
         }
     };
+    auto chunk_on = [&](uint64_t live, int j) { return ((live >> (j >> p.slot_shift)) & 1) != 0; };
 
     if (warp < kSoftmaxWarps) {
         // ================= softmax warpgroups =================
@@ -328,7 +334,12 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                         float* slot = xch + (j & 1) * 512;
                         slot[sub * 256 + r] = chunk_max;
                         wg_sync();
-                        if (sub == 0) cmax[j * 128] = (uint16_t)pack_bf16x2(sm::max_nan(chunk_max, slot[256 + r]), 0.0f);
+                        if (sub == 0) {
+                            uint16_t* e = cmax + (j >> p.slot_shift) * 128;
+                            float cm = sm::max_nan(chunk_max, slot[256 + r]);
+                            if ((j & ((1 << p.slot_shift) - 1)) != 0) cm = sm::max_nan(cm, __uint_as_float((uint32_t)*e << 16));
+                            *e = (uint16_t)pack_bf16x2(cm, 0.0f);
+                        }
                         chunk_max = -INFINITY;
                     }
                 }
@@ -344,13 +355,14 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 const uint32_t r2 = pack_bf16x2(__uint_as_float(r1 << 16) * p.scaling, 0.0f);
                 row_max = __uint_as_float(r2 << 16);
             }
-            uint64_t my_live = my_n >= 64 ? ~0ull : ((1ull << my_n) - 1);
+            uint64_t my_live = ~0ull;
             if (use_table) {
-                for (int j = 0; j < my_n; ++j) {
-                    const float cm = __uint_as_float((uint32_t)cmax[j * 128] << 16);
+                const int n_slots = ((my_n - 1) >> p.slot_shift) + 1;
+                for (int s = 0; s < n_slots; ++s) {
+                    const float cm = __uint_as_float((uint32_t)cmax[s * 128] << 16);
                     const bool counts = row_live && !(cm - row_max < -110.0f);
                     const unsigned any = __ballot_sync(0xFFFFFFFFu, counts);
-                    if (lane == 0 && any) atomicOr(&live_words[2 * wg + (j >> 5)], 1u << (j & 31));
+                    if (lane == 0 && any) atomicOr(&live_words[2 * wg + (s >> 5)], 1u << (s & 31));
                 }
                 if (r == 0) atomicOr(&live_words[2 * wg], 1u);  // (a warpgroup always walks its first chunk: the output accumulator gets written)
                 mbar_arrive(&scan_done[wg]);
@@ -358,9 +370,13 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 my_live = (uint64_t)live_words[2 * wg] | ((uint64_t)live_words[2 * wg + 1] << 32);
             }
             // ---- pass B: row sum of expf(x - max), the per-block sums added in K4a's order (sm::sum_layout): blocks in order, or
-            // butterfly-reduced groups of 8 added in order.  Both threads of a row add all four sums of a chunk, in the same order.
+            // butterfly-reduced groups of 8 or 32 added in order.  Layouts 0 / 1: both threads of a row add all four sums of a
+            // chunk, in the same order.  Layout 2: a group of 32 blocks is E + O (mxq_softmax_core.cuh), and the sub-0 thread owns
+            // exactly the even blocks of a row, the sub-1 thread the odd ones -- each builds its half alone, and the two threads
+            // exchange only the halves, once per group.
             {
                 float acc = 0.0f, a0 = 0.0f, a1 = 0.0f, a2 = 0.0f, a3 = 0.0f;
+                float n[8] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f, 0.0f};  // layout 2: this thread's first tree level of the open group
                 bool have_acc = false;
                 auto add_block = [&](int t, float s) {
                     if (p.layout == 0) {
@@ -382,14 +398,15 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                     }
                 };
                 for (int j = 0; j < my_n; ++j) {
-                    if (!((my_live >> j) & 1)) {  // every block of the chunk sums to +0 for every row of the warpgroup
+                    const bool walked = chunk_on(my_live, j);
+                    if (!walked && p.layout != 2) {  // every block of the chunk sums to +0 for every row of the warpgroup
 #pragma unroll
                         for (int bl = 0; bl < 4; ++bl) add_block(4 * j + bl, 0.0f);
                         continue;
                     }
-                    float mine[2];
+                    float mine[2] = {0.0f, 0.0f};
 #pragma unroll 1
-                    for (int hf = 0; hf < 2; ++hf) {
+                    for (int hf = 0; hf < 2 && walked; ++hf) {
                         uint32_t v[32];
                         take_ab(v);
                         const int t = 4 * j + 2 * hf + sub;
@@ -402,6 +419,26 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                         }
                         mine[hf] = s;
                     }
+                    if (p.layout == 2) {
+                        // blocks 4c + 2 hf + sub of the group (c = j & 7) are leaves 2c + hf of this thread's half; the first tree
+                        // level adds leaves i and i + 8.  Unvisited leaves (skipped chunks, the ragged tail, a half-filled last
+                        // group) stay +0, and every sum is >= +0, so adding them is exact.
+                        const int c4 = j & 3;
+                        n[0] += c4 == 0 ? mine[0] : 0.0f; n[1] += c4 == 0 ? mine[1] : 0.0f;
+                        n[2] += c4 == 1 ? mine[0] : 0.0f; n[3] += c4 == 1 ? mine[1] : 0.0f;
+                        n[4] += c4 == 2 ? mine[0] : 0.0f; n[5] += c4 == 2 ? mine[1] : 0.0f;
+                        n[6] += c4 == 3 ? mine[0] : 0.0f; n[7] += c4 == 3 ? mine[1] : 0.0f;
+                        if ((j & 7) == 7 || j == my_n - 1) {
+                            const float half = sm::butterfly8(n[0], n[1], n[2], n[3], n[4], n[5], n[6], n[7]);
+                            float* slot = xch + ((j >> 3) & 1) * 512;
+                            slot[sub * 256 + r] = half;
+                            wg_sync();
+                            acc = acc + (half + slot[(sub ^ 1) * 256 + r]);  // E + O; (acc starts at +0: exact for group 0)
+#pragma unroll
+                            for (int i = 0; i < 8; ++i) n[i] = 0.0f;
+                        }
+                        continue;
+                    }
                     float* slot = xch + (j & 1) * 512;
                     slot[sub * 256 + r] = mine[0];
                     slot[sub * 256 + 128 + r] = mine[1];
@@ -412,7 +449,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                     add_block(4 * j + 2, sub ? o1 : mine[1]);
                     add_block(4 * j + 3, sub ? mine[1] : o1);
                 }
-                if (p.layout != 0 && ((4 * my_n) & 7) != 0) {  // a half-filled last group (the rest of it: hidden blocks, sum 0)
+                if (p.layout == 1 && ((4 * my_n) & 7) != 0) {  // a half-filled last group (the rest of it: hidden blocks, sum 0)
                     const float g = ((a0 + 0.0f) + (a2 + 0.0f)) + ((a1 + 0.0f) + (a3 + 0.0f));
                     acc = have_acc ? acc + g : g;
                 }
@@ -421,7 +458,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
             // ---- pass C: the codes and scales of P, into the operand tile of the second contraction
             bool p_started = false;
             for (int j = 0; j < my_n; ++j) {
-                if (!((my_live >> j) & 1)) {  // +0 codes for the whole chunk: nothing for the tensor core to add
+                if (!chunk_on(my_live, j)) {  // +0 codes for the whole chunk: nothing for the tensor core to add
                     if (dump_codes != nullptr) {
                         const int sc = sm::dead_block_scale<ELEM>(row_max, row_sum);
                         dump_zero(4 * j + sub, sc);
@@ -529,7 +566,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                     need = live[0] | live[1];
                 }
                 for (int j = 0; j < n_cta; ++j) {
-                    if (!((need >> j) & 1)) continue;
+                    if (!chunk_on(need, j)) continue;
                     mbar_wait(&k_empty[ks], kph ^ 1);
                     mbar_arrive_expect_tx(&k_full[ks], TILE_BYTES);
                     tma_load_3d(&map_k, &k_full[ks], smem + Smem::OFF_K + ks * TILE_BYTES, 0, j * KC, bhk);
@@ -571,7 +608,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
             __syncwarp();
 #pragma unroll
             for (int wg = 0; wg < TILES; ++wg) {
-                if (!active[wg] || jj >= nv[wg] || !((live[wg] >> jj) & 1)) continue;
+                if (!active[wg] || jj >= nv[wg] || !chunk_on(live[wg], jj)) continue;
                 mbar_wait(&p_full[wg], pfull_par[wg]);
                 pfull_par[wg] ^= 1;
                 tc_fence_after();
@@ -600,13 +637,13 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
             if (pass == 1) {
                 live_chunks(live);
 #pragma unroll
-                for (int wg = 0; wg < TILES; ++wg) {
-                    const uint64_t m = live[wg] & (nv[wg] >= 64 ? ~0ull : ((1ull << nv[wg]) - 1));
-                    last_live[wg] = m ? 63 - __clzll((long long)m) : -1;
+                for (int wg = 0; wg < TILES; ++wg) {  // the last chunk below nv[wg] of the last live slot (a live slot holds one)
+                    const int s = live[wg] ? 63 - __clzll((long long)live[wg]) : -1;
+                    last_live[wg] = s < 0 ? -1 : min(nv[wg] - 1, ((s + 1) << p.slot_shift) - 1);
                 }
             }
             for (int j = 0; j < n_cta; ++j) {
-                if (pass > 0 && !(((live[0] | live[1]) >> j) & 1)) continue;
+                if (pass > 0 && !chunk_on(live[0] | live[1], j)) continue;
                 mbar_wait(&k_full[ks], kph);
                 mbar_wait(&ksf_full[ks], kph);
                 tc_fence_after();
@@ -620,7 +657,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 for (int hf = 0; hf < 2; ++hf) {
 #pragma unroll
                     for (int wg = 0; wg < TILES; ++wg) {
-                        if (!active[wg] || j >= nv[wg] || (pass > 0 && !((live[wg] >> j) & 1))) continue;
+                        if (!active[wg] || j >= nv[wg] || (pass > 0 && !chunk_on(live[wg], j))) continue;
                         uint32_t tm_s;
                         uint64_t* full_bar;
                         if (pass < 2) {  // two tiles per warpgroup inside its output accumulator: run one tile ahead of the softmax threads
@@ -694,7 +731,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 need = live[0] | live[1];
             }
             for (int j = 0; j < n_cta; ++j) {
-                if (!((need >> j) & 1)) continue;
+                if (!chunk_on(need, j)) continue;
                 uint32_t kw[4], vw[4];
                 load_k(j, kw);
                 if (pass == 2) {
@@ -746,13 +783,13 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
         snprintf(msg, msg_len, "operands must be 8-bit floating-point containers and the probabilities a floating-point element type");
         return MXQ_ERR_UNSUPPORTED_SHAPE;
     }
+    if (a->kv_len > MXQ_FLASH_MAX_KV) {
+        snprintf(msg, msg_len, "kv_len %lld > %d", (long long)a->kv_len, MXQ_FLASH_MAX_KV);
+        return MXQ_ERR_UNSUPPORTED_SHAPE;
+    }
     const bool masked = a->causal || a->mask != nullptr;
     const int tpr = (int)(a->kv_len / 32);
     const int layout = sm::sum_layout(tpr, masked);
-    if (layout == 2) {
-        snprintf(msg, msg_len, "row sums of %d blocks (%s) are added in an order this kernel does not reproduce", tpr, masked ? "masked" : "unmasked");
-        return MXQ_ERR_UNSUPPORTED_SHAPE;
-    }
     auto al16 = [](const void* ptr) { return ((uintptr_t)ptr % 16) == 0; };
     if (!al16(a->q_codes) || !al16(a->k_codes) || !al16(a->vt_codes) || ((uintptr_t)a->q_scales % 4) || ((uintptr_t)a->k_scales % 4) ||
         ((a->kv_len % KC) == 0 && ((uintptr_t)a->vt_scales % 4)) ||
@@ -783,6 +820,8 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
     p.causal_offset = (int)(a->kv_len - a->q_len);
     p.skip_hidden_chunks = p.causal;  // (an explicit mask is data: every chunk is read)
     p.layout = layout;
+    const int n_chunks = (int)((a->kv_len + KC - 1) / KC);
+    while ((64 << p.slot_shift) < n_chunks) ++p.slot_shift;
     p.scaling = a->scaling;
     // the probabilities travel as E4M3 bytes (exact for every fp6 / fp4 value) unless they ARE e5m2
     const int p_format = a->p_elem == MXQ_ELEM_E5M2 ? MXQ_OPERAND_E5M2_BYTES : MXQ_OPERAND_E4M3_BYTES;

@@ -349,7 +349,8 @@ class _MXAttentionMixin:
         elif q_len > 1 and getattr(self, "is_causal", True):
             causal = True  # mask creation was skipped because the attention function is expected to apply is_causal itself
         dropout = self.training and getattr(self, "attention_dropout", 0.0)
-        if not dropout and 32 == qc.query_config.block_size == qc.key_config.block_size == qc.value_config.block_size:
+        if not dropout and 32 == qc.query_config.block_size == qc.key_config.block_size == qc.value_config.block_size \
+                and not attention_ops.chain_is_faster(q_mx.shape[0], k_one.shape[1], q_len, kv_len, mask is not None or causal):
             # K4b: both contractions, the softmax chain and the quantization of P as one kernel -- the scores and P never reach HBM;
             # key / value heads are read in place by the query heads that share them (no repeated copies)
             out = attention_ops.flash_attention(q_mx, k_one, vt_one, scaling, mask, causal, pc.elem_dtype, pc.block_size)
