@@ -283,6 +283,15 @@ MXQ_API int mxq_gemm_bf16(const void *a, int64_t lda, int64_t a_batch_stride, co
  *   p_elem   : element type of P (any floating-point mxq_elem_t), flags: MXQ_FLAG_*
  * MXQ_ERR_UNSUPPORTED_SHAPE unless head_dim == 128, kv_len % 32 == 0, q_len <= kv_len <= MXQ_FLASH_MAX_KV (masked or not).  Rows
  * of any length add their block sums in mxq_softmax_quantize's order, including the lengths that entry point itself refuses.
+ *   kv_pitch : 0, or the key capacity of K / V buffers of which only the first kv_len keys exist (a KV cache read in place):
+ *              k_codes [batch, kv_heads, kv_pitch, 128], k_scales [.., kv_pitch, 4], vt_codes [batch, kv_heads, 128, kv_pitch],
+ *              vt_scales [.., kv_pitch / 32]; 1 <= q_len <= kv_len <= kv_pitch <= MXQ_FLASH_MAX_KV and kv_pitch % 128 == 0, else
+ *              MXQ_ERR_INVALID.  kv_len may be any value.  With n = kv_len rounded up to a multiple of 128, the result is, bit
+ *              for bit, that of kv_pitch 0 on contiguous copies of the first n keys (zero codes past kv_len) with causal 0 and the
+ *              mask mask' = the given mask (or zeros) with -inf on every key the causal rule hides and on every key >= kv_len
+ *              (no mask at all when none is given, causal is 0 and kv_len == n).  p_codes / p_scales are then [.., n] /
+ *              [.., n / 32].  No K code, K scale or V code at a position >= kv_len is read, nor the V scale of a block wholly
+ *              past it.
  */
 #define MXQ_FLASH_MAX_KV 131072
 typedef struct {
@@ -296,6 +305,7 @@ typedef struct {
     int p_elem /* mxq_elem_t */; unsigned flags /* MXQ_FLAG_* */;
     void *out; int64_t out_batch_stride, out_head_stride, out_row_stride;
     void *p_codes; uint8_t *p_scales;
+    int64_t kv_pitch;
 } mxq_attention_args_t;
 MXQ_API int mxq_flash_attention(const mxq_attention_args_t *args, int device, void *stream);
 
@@ -427,6 +437,7 @@ MXQ_API int mxq_rope_quantize_kv(const mxq_rope_quantize_kv_args_t *args, int de
 #define MXQ_ERR_CUDA 3
 
 MXQ_API const char *mxq_last_error(void);
+/* ABI version: 5 (mxq_attention_args_t.kv_pitch) */
 MXQ_API int mxq_version(void);
 /* compiled-for architecture as an integer (1000 for sm_100a) -- lets the host refuse to run a
  * library that was built for something else instead of failing inside a launch. */

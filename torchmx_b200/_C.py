@@ -14,7 +14,7 @@ HP_BF16, HP_F32 = 0, 1
 FLAG_HW_EXACT = 1
 FLAG_OPERAND_LAYOUT = 2
 GEMM_B_STATIC, GEMM_WIDE_TILES, GEMM_NO_PDL, GEMM_NO_MXF4 = 1, 2, 4, 8
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_DIMS = 6
 
 EXPORTS = ("mxq_quantize", "mxq_dequantize", "mxq_dequantize_strided", "mxq_gemm", "mxq_gemm_dequant", "mxq_gemm_bf16", "mxq_transcode_to_e4m3", "mxq_pack_operand", "mxq_unpack_operand",
@@ -81,6 +81,7 @@ class AttentionArgs(ctypes.Structure):
         ("p_elem", ctypes.c_int), ("flags", ctypes.c_uint),
         ("out", ctypes.c_void_p), ("out_batch_stride", ctypes.c_int64), ("out_head_stride", ctypes.c_int64), ("out_row_stride", ctypes.c_int64),
         ("p_codes", ctypes.c_void_p), ("p_scales", ctypes.c_void_p),
+        ("kv_pitch", ctypes.c_int64),
     ]
 
 

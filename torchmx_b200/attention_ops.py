@@ -105,21 +105,34 @@ def _byte_operand(t: MXTensor):
 
 
 def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: float, mask: Optional[torch.Tensor], causal: bool,
-                    p_elem_dtype: dtypes.DType, p_block_size: int = 32, return_probs: bool = False):
+                    p_elem_dtype: dtypes.DType, p_block_size: int = 32, return_probs: bool = False, kv_len: Optional[int] = None):
     """The reference's MX attention (torchmx/layers/mx_llama_attention.py:195-243) in one launch.
 
     q_mx [b, h, q, 128] and k_mx [b, h_kv, kv, 128] quantized along head_dim, vt_mx [b, h_kv, 128, kv] = V quantized along the
     key axis (the reference's quantize-the-transpose), all contiguous with block size 32; mask: None or additive bf16
     broadcastable to [b, h, q, kv].  Returns the attention output already in the [b, q, h, 128] layout the reference transposes
     to next (bf16) -- plus the MXTensor of P when `return_probs` -- or None when the kernel does not apply (the caller then
-    runs the K3 -> K4a -> K3 chain)."""
+    runs the K3 -> K4a -> K3 chain).
+
+    kv_len: None, or the number of keys that exist in K / Vt buffers of a capacity (a multiple of 128) -- a KV cache read in
+    place.  Then kv_len may be anything from q_len to the capacity, mask (if any) covers >= kv_len keys, and the result is
+    that of the call without kv_len on `ragged_operands(...)` (P then has n = ceil128(kv_len) keys)."""
     if not _FLASH or p_block_size != 32 or p_elem_dtype == dtypes.int8 or q_mx.dim() != 4 or k_mx.dim() != 4 or vt_mx.dim() != 4:
         return None
     b, h, q_len, d = q_mx.shape
-    hk, kv_len = k_mx.shape[1], k_mx.shape[2]
-    if d != 128 or k_mx.shape != (b, hk, kv_len, d) or vt_mx.shape != (b, hk, d, kv_len) or h % hk or kv_len % 32 or kv_len < q_len or q_len == 0:
+    hk, pitch = k_mx.shape[1], k_mx.shape[2]
+    ragged = kv_len is not None
+    if not ragged:
+        kv_len, n = pitch, pitch
+        if pitch % 32:
+            return None
+    else:
+        n = -(-kv_len // 128) * 128
+        if pitch % 128 or kv_len > pitch:
+            return None
+    if d != 128 or k_mx.shape != (b, hk, pitch, d) or vt_mx.shape != (b, hk, d, pitch) or h % hk or kv_len < q_len or q_len == 0:
         return None
-    if kv_len > MAX_FLASH_KV:
+    if pitch > MAX_FLASH_KV:
         return None
     ops = [_byte_operand(t) for t in (q_mx, k_mx, vt_mx)]
     if any(o is None for o in ops):
@@ -138,10 +151,11 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
         [(c.data_ptr(), f, s.data_ptr()) for c, f, s in ops]
     a.batch, a.heads, a.kv_heads, a.q_len, a.kv_len, a.head_dim = b, h, hk, q_len, kv_len, d
     a.scaling, a.causal = float(scaling), 1 if causal else 0
+    a.kv_pitch = pitch if ragged else 0
     # One query position (decode) with grouped-query heads: the query heads that share a key / value head become the ROWS of one
     # query tile ([b, h, 1, d] is [b, h_kv, groups, d] in memory), so a CTA works on `groups` live rows instead of one and the grid
     # shrinks by that factor.  Same rows, same keys, same arithmetic per row; the mask row is shared by the group.
-    grouped = q_len == 1 and h > hk and not causal and (mask is None or mask.shape[1] == 1)
+    grouped = q_len == 1 and h > hk and not causal and (mask is None or mask.shape[1] == 1) and (not ragged or kv_len >= h // hk)
     if grouped:
         a.heads, a.q_len, a.mask_stride_q = hk, h // hk, 0
     a.p_elem = dtypes.ELEM_ID[p_elem_dtype.name]
@@ -153,8 +167,8 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
     probs = None
     if return_probs:
         is_fp4 = p_elem_dtype == dtypes.float4_e2m1
-        p_codes = torch.empty((b, h, q_len, kv_len // 2 if is_fp4 else kv_len), dtype=torch.uint8, device=dev)
-        p_scales = torch.empty((b, h, q_len, kv_len // 32), dtype=torch.uint8, device=dev)
+        p_codes = torch.empty((b, h, q_len, n // 2 if is_fp4 else n), dtype=torch.uint8, device=dev)
+        p_scales = torch.empty((b, h, q_len, n // 32), dtype=torch.uint8, device=dev)
         a.p_codes, a.p_scales = p_codes.data_ptr(), p_scales.data_ptr()
         probs = MXTensor(p_scales, p_codes, p_elem_dtype, 32, torch.bfloat16)
     rc = _C.lib().mxq_flash_attention(a, dev.index, _stream_ptr(q_mx._data))
@@ -163,3 +177,30 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
     _C.check(rc, "mxq_flash_attention")
     stats["flash_attention"] += 1
     return (out, probs) if return_probs else out
+
+
+def ragged_operands(k_mx: MXTensor, vt_mx: MXTensor, kv_len: int, q_len: int, mask: Optional[torch.Tensor], causal: bool):
+    """What `flash_attention(..., kv_len=kv_len)` computes, as operands of the call without kv_len (and of the K3 -> K4a -> K3
+    chain): (K, Vt, mask') with n = ceil128(kv_len) keys.  K / Vt are contiguous copies of the first n keys of the capacity
+    buffers with zero codes at positions >= kv_len, the neutral scale 127 on those keys and on the V blocks wholly past kv_len;
+    mask' is the additive bf16 `mask` (or zeros) with -inf on every key >= kv_len and, when `causal`, on every key j > q +
+    (kv_len - q_len) -- or None when there is no mask, causal is off and kv_len == n.  O(kv_len) copies."""
+    n = -(-kv_len // 128) * 128
+    k_codes, k_scales = k_mx._data[:, :, :n].clone(), k_mx._scale_e8m0[:, :, :n].clone()
+    vt_codes, vt_scales = vt_mx._data[..., :n].clone(), vt_mx._scale_e8m0[..., :n // 32].clone()
+    k_codes[:, :, kv_len:] = 0
+    k_scales[:, :, kv_len:] = 127
+    vt_codes[..., kv_len:] = 0
+    vt_scales[..., -(-kv_len // 32):] = 127
+    k_n = MXTensor(k_scales, k_codes, k_mx._elem_dtype, 32, k_mx._orig_dtype)
+    vt_n = MXTensor(vt_scales, vt_codes, vt_mx._elem_dtype, 32, vt_mx._orig_dtype)
+    if mask is None and not causal and kv_len == n:
+        return k_n, vt_n, None
+    dev = k_codes.device
+    shape = (1, 1, q_len) if mask is None else (*mask.shape[:2], q_len)
+    mask_n = torch.full((*shape, n), float("-inf"), dtype=torch.bfloat16, device=dev)
+    mask_n[..., :kv_len] = 0 if mask is None else mask[..., :kv_len]
+    if causal:
+        hidden = torch.ones(q_len, n, dtype=torch.bool, device=dev).triu_(kv_len - q_len + 1)
+        mask_n.masked_fill_(hidden, float("-inf"))
+    return k_n, vt_n, mask_n

@@ -88,7 +88,7 @@ int waves_override() { static int v = env_int("MXQ_WAVES"); return v > 0 ? v : 0
 extern "C" {
 
 const char* mxq_last_error(void) { return g_err; }
-int mxq_version(void) { return 4; }
+int mxq_version(void) { return 5; }
 int mxq_arch(void) { return 1000; }
 
 int mxq_quantize(const void* src, int src_dtype, int64_t n_blocks, int block_size, int elem, unsigned flags, void* codes, uint8_t* scales,
@@ -303,6 +303,9 @@ int mxq_flash_attention(const mxq_attention_args_t* a, int device, void* stream)
     if (!a->q_codes || !a->q_scales || !a->k_codes || !a->k_scales || !a->vt_codes || !a->vt_scales || !a->out)
         return fail(MXQ_ERR_INVALID, "mxq_flash_attention: null pointer");
     if ((a->p_codes == nullptr) != (a->p_scales == nullptr)) return fail(MXQ_ERR_INVALID, "mxq_flash_attention: p_codes and p_scales go together");
+    if (a->kv_pitch < 0 || (a->kv_pitch > 0 && (a->kv_pitch % 128 || a->kv_pitch > MXQ_FLASH_MAX_KV || a->kv_len > a->kv_pitch || a->q_len > a->kv_len)))
+        return fail(MXQ_ERR_INVALID, "mxq_flash_attention: kv_pitch %lld must be 0 or a multiple of 128 with q_len %lld <= kv_len %lld <= kv_pitch <= %d",
+                    (long long)a->kv_pitch, (long long)a->q_len, (long long)a->kv_len, MXQ_FLASH_MAX_KV);
     DeviceScope scope(device);
     if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_flash_attention: selecting device");
     char msg[400] = "";

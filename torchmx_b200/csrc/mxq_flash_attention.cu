@@ -31,6 +31,11 @@
 // pass A records the largest score of every (row, slot) and passes B / C skip the slots that are dead for a whole tile.  A slot
 // is 2^slot_shift consecutive chunks, as few as keep a row at 64 slots (one chunk per slot up to 8192 keys).
 // The key axis may be any multiple of 32 up to MXQ_FLASH_MAX_KV (a ragged last chunk is zero-filled by TMA and hidden).
+// RAGGED instantiations (kv_pitch > 0) read the first kv_valid keys of K / V buffers pitched for kv_pitch keys -- a KV cache read
+// in place at whatever length it has.  They compute exactly what the kernel computes on contiguous copies of the first
+// n = ceil128(kv_valid) keys (zero codes in the tail) with causal off and the mask mask' = caller's mask (or zeros), -inf on every
+// key the causal rule hides and on every key >= kv_valid: here kv_len is n, and the -inf keys are added in scores_of.  Nothing at
+// or past kv_valid is read: the tensor maps end there (TMA zero-fills), and the scale loader feeds the neutral scale 127.
 #include <cstring>
 
 #include "mxq_softmax_core.cuh"
@@ -104,6 +109,7 @@ struct Params {
     uint32_t idesc_qk, idesc_pv;
     uint32_t flags;
     int q_tiles;
+    int kv_valid, hide_offset, kv_pitch;  // RAGGED: keys that exist; a row q sees keys < min(kv_valid, q + hide_offset + 1); key pitch
 };
 
 __device__ __forceinline__ uint32_t to_e4m3_pair(uint32_t h2) {  // f16x2 -> two e4m3 bytes (exact for every fp6 / fp4 value)
@@ -137,7 +143,7 @@ __device__ __forceinline__ void container_bytes(const uint32_t (&out)[(ELEM == M
     }
 }
 
-template <int ELEM, bool TABLE, int TILES>
+template <int ELEM, bool TABLE, int TILES, bool RAGGED>
 __global__ void __launch_bounds__(Cfg<TILES>::kThreads, TILES == 2 ? 1 : 2)
 mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k, const __grid_constant__ CUtensorMap map_v, const Params p) {
     using C = Cfg<TILES>;
@@ -244,6 +250,7 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
         const int my_n = nv[wg];
         const uint32_t tm_lane = tmem_base + ((uint32_t)(quad * 32) << 16);
         const uint16_t* mrow = (TABLE && p.mask != nullptr && row_live) ? p.mask + (int64_t)b * p.mask_sb + (int64_t)h * p.mask_sh + (int64_t)q * p.mask_sq : nullptr;
+        const int row_lim = RAGGED ? min(p.kv_valid, q + p.hide_offset + 1) : 0;  // RAGGED: the keys of mask' that are not -inf
         const int tpr = p.kv_len / 32;
         const bool hw_exact = (p.flags & MXQ_FLAG_HW_EXACT) != 0;
         uint8_t* p_tile = smem + Smem::OFF_P + wg * TILE_BYTES + r * 128;
@@ -289,7 +296,23 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
 #pragma unroll
             for (int i = 0; i < 16; ++i) w[i] = pack_bf16x2(__uint_as_float(raw[2 * i]), __uint_as_float(raw[2 * i + 1]));
             sm::scale_round(w, p.scaling, x);
-            if (mrow != nullptr) {
+            if constexpr (RAGGED) {  // + mask': the caller's mask is read only at the keys it does not replace by -inf
+                const int hv = row_lim - t * 32;
+                if (mrow != nullptr || hv < 32) {
+                    uint32_t mw[16];
+                    if (mrow != nullptr && hv >= 32) {
+                        sm::load_mask(mrow + t * 32, p.mask_vec != 0, mw);
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) {
+                            const uint32_t m0 = 2 * i < hv ? (mrow != nullptr ? mrow[t * 32 + 2 * i] : 0u) : 0xFF80u;  // bf16 -inf
+                            const uint32_t m1 = 2 * i + 1 < hv ? (mrow != nullptr ? mrow[t * 32 + 2 * i + 1] : 0u) : 0xFF80u;
+                            mw[i] = m0 | (m1 << 16);
+                        }
+                    }
+                    sm::add_mask(x, mw);
+                }
+            } else if (mrow != nullptr) {
                 uint32_t mw[16];
                 sm::load_mask(mrow + t * 32, p.mask_vec != 0, mw);
                 sm::add_mask(x, mw);
@@ -715,12 +738,19 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
             }
             publish(qsf_full);
         }
-        const uint32_t* ksrc = reinterpret_cast<const uint32_t*>(p.k_sf) + (int64_t)bhk * p.kv_len;
-        const int vld = p.kv_len / 32;  // scale bytes per channel row of V^T
+        const uint32_t* ksrc = reinterpret_cast<const uint32_t*>(p.k_sf) + (int64_t)bhk * (RAGGED ? p.kv_pitch : p.kv_len);
+        const int vld = (RAGGED ? p.kv_pitch : p.kv_len) / 32;  // scale bytes per channel row of V^T
         const uint8_t* vsrc = p.v_sf + (int64_t)bhk * HD * vld;
         auto load_k = [&](int j, uint32_t (&w)[4]) {
 #pragma unroll
-            for (int i = 0; i < 4; ++i) w[i] = __ldg(ksrc + min(j * KC + i * 32 + lane, p.kv_len - 1));  // (keys past kv_len: zero codes, hidden)
+            for (int i = 0; i < 4; ++i) {
+                if constexpr (RAGGED) {  // keys past kv_valid: zero codes (TMA fill) times the neutral scale
+                    const int key = j * KC + i * 32 + lane;
+                    w[i] = key < p.kv_valid ? __ldg(ksrc + key) : 0x7F7F7F7Fu;
+                } else {
+                    w[i] = __ldg(ksrc + min(j * KC + i * 32 + lane, p.kv_len - 1));  // (keys past kv_len: zero codes, hidden)
+                }
+            }
         };
         uint32_t ks = 0, kph = 0, vs = 0, vph = 0;
         uint64_t need = ~0ull;
@@ -735,16 +765,17 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
                 uint32_t kw[4], vw[4];
                 load_k(j, kw);
                 if (pass == 2) {
-                    if ((vld & 3) == 0) {
+                    const int vb = RAGGED ? (p.kv_valid + 31) / 32 : vld;  // V scale blocks that hold a key
+                    if ((vld & 3) == 0 && (!RAGGED || 4 * j + 4 <= vb)) {
 #pragma unroll
                         for (int i = 0; i < 4; ++i) vw[i] = __ldg(reinterpret_cast<const uint32_t*>(vsrc + (int64_t)(i * 32 + lane) * vld + 4 * j));
-                    } else {  // ragged kv_len: a channel's scale row is not a whole number of words
+                    } else {  // ragged kv_len (a channel's scale row is not a whole number of words), or the chunk reaching past kv_valid
 #pragma unroll
                         for (int i = 0; i < 4; ++i) {
                             const uint8_t* row = vsrc + (int64_t)(i * 32 + lane) * vld;
                             uint32_t w = 0;
 #pragma unroll
-                            for (int bb = 0; bb < 4; ++bb) w |= (uint32_t)(4 * j + bb < vld ? __ldg(row + 4 * j + bb) : 127) << (8 * bb);
+                            for (int bb = 0; bb < 4; ++bb) w |= (uint32_t)(4 * j + bb < vb ? __ldg(row + 4 * j + bb) : 127) << (8 * bb);
                             vw[i] = w;
                         }
                     }
@@ -775,7 +806,10 @@ mx_flash_attention_kernel(const __grid_constant__ CUtensorMap map_q, const __gri
 int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream_t stream, char* msg, size_t msg_len) {
     using namespace fa;
     auto fmt_ok = [](int f) { return f == MXQ_OPERAND_E4M3_BYTES || f == MXQ_OPERAND_E5M2_BYTES; };
-    if (a->head_dim != HD || a->kv_len % 32 || a->kv_len < 32 || a->q_len < 1 || a->kv_len < a->q_len || a->heads % a->kv_heads) {
+    const bool ragged = a->kv_pitch > 0;  // (the C entry checked 1 <= q_len <= kv_len <= kv_pitch <= MXQ_FLASH_MAX_KV, kv_pitch % 128 == 0)
+    // the key axis the kernel walks: kv_len, or in the ragged mode n = ceil128(kv_len) keys of which the tail is hidden
+    const int64_t kv_n = ragged ? (a->kv_len + KC - 1) / KC * KC : a->kv_len;
+    if (a->head_dim != HD || (!ragged && (a->kv_len % 32 || a->kv_len < 32)) || a->q_len < 1 || a->kv_len < a->q_len || a->heads % a->kv_heads) {
         snprintf(msg, msg_len, "needs head_dim == 128, kv_len %% 32 == 0, kv_len >= q_len, heads %% kv_heads == 0");
         return MXQ_ERR_UNSUPPORTED_SHAPE;
     }
@@ -787,12 +821,13 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
         snprintf(msg, msg_len, "kv_len %lld > %d", (long long)a->kv_len, MXQ_FLASH_MAX_KV);
         return MXQ_ERR_UNSUPPORTED_SHAPE;
     }
-    const bool masked = a->causal || a->mask != nullptr;
-    const int tpr = (int)(a->kv_len / 32);
+    // mask' of the ragged mode exists unless the caller gave no mask, causal is off and kv_len == n
+    const bool masked = a->causal || a->mask != nullptr || kv_n != a->kv_len;
+    const int tpr = (int)(kv_n / 32);
     const int layout = sm::sum_layout(tpr, masked);
     auto al16 = [](const void* ptr) { return ((uintptr_t)ptr % 16) == 0; };
     if (!al16(a->q_codes) || !al16(a->k_codes) || !al16(a->vt_codes) || ((uintptr_t)a->q_scales % 4) || ((uintptr_t)a->k_scales % 4) ||
-        ((a->kv_len % KC) == 0 && ((uintptr_t)a->vt_scales % 4)) ||
+        ((ragged || (a->kv_len % KC) == 0) && ((uintptr_t)a->vt_scales % 4)) ||
         !al16(a->out) || (a->out_batch_stride % 8) || (a->out_head_stride % 8) || (a->out_row_stride % 8) || (a->p_codes && !al16(a->p_codes))) {
         snprintf(msg, msg_len, "misaligned operand");
         return MXQ_ERR_UNSUPPORTED_SHAPE;
@@ -801,10 +836,11 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
     const int tiles = a->q_len <= QT ? 1 : 2;  // query tiles per CTA: one (two CTAs per SM) when a (batch, head) has at most 128 query rows
     const int64_t q_tiles = (a->q_len + tiles * QT - 1) / (tiles * QT);
     if (bh * q_tiles > 0x7FFFFFFF || a->q_len > 0x3FFFFFFF || a->kv_len > 0x3FFFFFFF) { snprintf(msg, msg_len, "extent too large"); return MXQ_ERR_UNSUPPORTED_SHAPE; }
+    const int64_t pitch = ragged ? a->kv_pitch : a->kv_len;  // the maps end at kv_len: TMA zero-fills the keys past it
     CUtensorMap map_q, map_k, map_v;
     if (!cached_operand_map(&map_q, a->q_codes, HD, a->q_len, bh, HD, a->q_len * HD, 128, a->q_format, device) ||
-        !cached_operand_map(&map_k, a->k_codes, HD, a->kv_len, bhk, HD, a->kv_len * HD, 128, a->k_format, device) ||
-        !cached_operand_map(&map_v, a->vt_codes, a->kv_len, HD, bhk, a->kv_len, (int64_t)HD * a->kv_len, 128, a->v_format, device)) {
+        !cached_operand_map(&map_k, a->k_codes, HD, a->kv_len, bhk, HD, pitch * HD, 128, a->k_format, device) ||
+        !cached_operand_map(&map_v, a->vt_codes, a->kv_len, HD, bhk, pitch, (int64_t)HD * pitch, 128, a->v_format, device)) {
         snprintf(msg, msg_len, "cuTensorMapEncodeTiled failed");
         return MXQ_ERR_CUDA;
     }
@@ -815,12 +851,16 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
     p.mask_vec = a->mask && ((uintptr_t)a->mask % 16 == 0) && (a->mask_stride_b % 8 == 0) && (a->mask_stride_h % 8 == 0) && (a->mask_stride_q % 8 == 0);
     p.out = (uint16_t*)a->out; p.out_sb = a->out_batch_stride; p.out_sh = a->out_head_stride; p.out_sq = a->out_row_stride;
     p.p_codes = (uint8_t*)a->p_codes; p.p_scales = a->p_scales;
-    p.batch = (int)a->batch; p.heads = (int)a->heads; p.kv_heads = (int)a->kv_heads; p.q_len = (int)a->q_len; p.kv_len = (int)a->kv_len;
-    p.causal = a->causal ? 1 : 0;
+    p.batch = (int)a->batch; p.heads = (int)a->heads; p.kv_heads = (int)a->kv_heads; p.q_len = (int)a->q_len; p.kv_len = (int)kv_n;
+    // ragged: causal off, the causal rule and the tail folded into mask' (hide_offset: a row q sees keys <= q + hide_offset)
+    p.causal = a->causal && !ragged ? 1 : 0;
     p.causal_offset = (int)(a->kv_len - a->q_len);
     p.skip_hidden_chunks = p.causal;  // (an explicit mask is data: every chunk is read)
     p.layout = layout;
-    const int n_chunks = (int)((a->kv_len + KC - 1) / KC);
+    p.kv_valid = (int)a->kv_len;
+    p.hide_offset = a->causal ? (int)(a->kv_len - a->q_len) : (int)a->kv_len;
+    p.kv_pitch = (int)pitch;
+    const int n_chunks = (int)((kv_n + KC - 1) / KC);
     while ((64 << p.slot_shift) < n_chunks) ++p.slot_shift;
     p.scaling = a->scaling;
     // the probabilities travel as E4M3 bytes (exact for every fp6 / fp4 value) unless they ARE e5m2
@@ -830,22 +870,26 @@ int launch_flash_attention(const mxq_attention_args_t* a, int device, cudaStream
     p.flags = a->flags;
     p.q_tiles = (int)q_tiles;
     const unsigned grid = (unsigned)(bh * q_tiles);
-#define MXQ_FA_LAUNCH(E, T, TL)                                                                                                     \
+#define MXQ_FA_LAUNCH(E, T, TL, R)                                                                                                  \
     {                                                                                                                               \
-        cudaError_t e = ensure_smem_attr((const void*)mx_flash_attention_kernel<E, T, TL>, SmemT<TL>::DYN_BYTES, device);            \
+        cudaError_t e = ensure_smem_attr((const void*)mx_flash_attention_kernel<E, T, TL, R>, SmemT<TL>::DYN_BYTES, device);         \
         if (e != cudaSuccess) { snprintf(msg, msg_len, "cudaFuncSetAttribute: %s", cudaGetErrorString(e)); return MXQ_ERR_CUDA; }   \
-        mx_flash_attention_kernel<E, T, TL><<<grid, Cfg<TL>::kThreads, SmemT<TL>::DYN_BYTES, stream>>>(map_q, map_k, map_v, p);      \
+        mx_flash_attention_kernel<E, T, TL, R><<<grid, Cfg<TL>::kThreads, SmemT<TL>::DYN_BYTES, stream>>>(map_q, map_k, map_v, p);   \
     }
+    // the ragged mode runs the table (mask) variant whenever mask' exists, with or without a caller's mask
+#define MXQ_FA_TILES(E, R)                                                                                                          \
+    if (tiles == 1) { if (R ? masked : a->mask != nullptr) MXQ_FA_LAUNCH(E, true, 1, R) else MXQ_FA_LAUNCH(E, false, 1, R) }          \
+    else { if (R ? masked : a->mask != nullptr) MXQ_FA_LAUNCH(E, true, 2, R) else MXQ_FA_LAUNCH(E, false, 2, R) }
 #define MXQ_FA_CASE(E)                                                                                                              \
     case E:                                                                                                                         \
-        if (tiles == 1) { if (a->mask != nullptr) MXQ_FA_LAUNCH(E, true, 1) else MXQ_FA_LAUNCH(E, false, 1) }                        \
-        else { if (a->mask != nullptr) MXQ_FA_LAUNCH(E, true, 2) else MXQ_FA_LAUNCH(E, false, 2) }                                   \
+        if (ragged) { MXQ_FA_TILES(E, true) } else { MXQ_FA_TILES(E, false) }                                                       \
         break;
     switch (a->p_elem) {
         MXQ_FA_CASE(MXQ_ELEM_E4M3) MXQ_FA_CASE(MXQ_ELEM_E3M2) MXQ_FA_CASE(MXQ_ELEM_E2M3) MXQ_FA_CASE(MXQ_ELEM_E2M1) MXQ_FA_CASE(MXQ_ELEM_E5M2)
     default: snprintf(msg, msg_len, "unknown element type %d", a->p_elem); return MXQ_ERR_INVALID;
     }
 #undef MXQ_FA_CASE
+#undef MXQ_FA_TILES
 #undef MXQ_FA_LAUNCH
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { snprintf(msg, msg_len, "launch (flash attention): %s", cudaGetErrorString(e)); return MXQ_ERR_CUDA; }

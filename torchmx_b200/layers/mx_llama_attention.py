@@ -14,7 +14,8 @@ past_key_values, **kwargs) -> (attn_output, attn_weights)`), not the 4.44 intern
 With HF's caches the KV cache stays in high precision (reference :186-187) and, with a full `QAttentionConfig`, the whole cache is
 quantized again at every forward.  With an `MXStaticCache` (torchmx_b200/kv_cache.py) and a full `QAttentionConfig` the cache holds
 the MX codes themselves: one launch (K5e) rotates, quantizes Q and appends only the new tokens' blocks, and the attention reads the
-cache in place -- the same codes, so the same logits as with a bf16 StaticCache.
+cache in place -- the same codes, so the same logits as with a bf16 StaticCache.  An `MXDynamicCache` works the same way with a
+cache that grows with the sequence: the attention reads its first L positions in place, at any length L.
 """
 from __future__ import annotations
 
@@ -26,7 +27,7 @@ from torch import nn
 
 from .. import attention_ops, glue_ops, mlp_ops, mx_gemm
 from ..config import QAttentionConfig, QLinearConfig
-from ..kv_cache import MXStaticCache
+from ..kv_cache import MXDynamicCache, MXStaticCache
 from ..mx_tensor import MXTensor
 from .mx_linear import MXInferenceLinear
 
@@ -334,13 +335,16 @@ class _MXAttentionMixin:
             vt_one = MXTensor.to_mx(value_states.transpose(2, 3).contiguous(), qc.value_config.elem_dtype, qc.value_config.block_size)
         return self._mx_attend(q_mx, k_one, vt_one, attention_mask, scaling, dtype)
 
-    def _mx_attend(self, q_mx: MXTensor, k_one: MXTensor, vt_one: MXTensor, attention_mask, scaling: float, dtype: torch.dtype) -> torch.Tensor:
+    def _mx_attend(self, q_mx: MXTensor, k_one: MXTensor, vt_one: MXTensor, attention_mask, scaling: float, dtype: torch.dtype,
+                   kv_len: Optional[int] = None) -> torch.Tensor:
         """the attention on MX operands: q_mx [bs, heads, q_len, head_dim], k_one [bs, kv_heads, kv_len, head_dim] and vt_one
-        [bs, kv_heads, head_dim, kv_len] (V quantized along the sequence) -> [bs, q_len, heads, head_dim]"""
+        [bs, kv_heads, head_dim, kv_len] (V quantized along the sequence) -> [bs, q_len, heads, head_dim].  With `kv_len`, k_one
+        / vt_one are the buffers of an MXDynamicCache, of which the first kv_len positions exist."""
         qc = self.qconfig
         groups = self.num_key_value_groups
         pc = qc.attention_weights_config
-        q_len, kv_len = q_mx.shape[-2], k_one.shape[-2]
+        ragged = kv_len is not None
+        q_len, kv_len = q_mx.shape[-2], (kv_len if ragged else k_one.shape[-2])
         mask, causal = None, False
         if attention_mask is not None:  # no matter the length, we just slice it (reference :218-220)
             mask = attention_mask[:, :, :, :kv_len]
@@ -349,13 +353,19 @@ class _MXAttentionMixin:
         elif q_len > 1 and getattr(self, "is_causal", True):
             causal = True  # mask creation was skipped because the attention function is expected to apply is_causal itself
         dropout = self.training and getattr(self, "attention_dropout", 0.0)
+        # a cache read in place walks n = ceil128(kv_len) keys, the tail past kv_len masked (attention_ops.ragged_operands)
+        n = -(-kv_len // 128) * 128 if ragged else kv_len
         if not dropout and 32 == qc.query_config.block_size == qc.key_config.block_size == qc.value_config.block_size \
-                and not attention_ops.chain_is_faster(q_mx.shape[0], k_one.shape[1], q_len, kv_len, mask is not None or causal):
+                and not attention_ops.chain_is_faster(q_mx.shape[0], k_one.shape[1], q_len, n, mask is not None or causal or n != kv_len):
             # K4b: both contractions, the softmax chain and the quantization of P as one kernel -- the scores and P never reach HBM;
             # key / value heads are read in place by the query heads that share them (no repeated copies)
-            out = attention_ops.flash_attention(q_mx, k_one, vt_one, scaling, mask, causal, pc.elem_dtype, pc.block_size)
+            out = attention_ops.flash_attention(q_mx, k_one, vt_one, scaling, mask, causal, pc.elem_dtype, pc.block_size,
+                                                kv_len=kv_len if ragged else None)
             if out is not None:
                 return out
+        if ragged:  # the same result from the chain, on copies of the first n positions with the tail and the causal rule in the mask
+            k_n, vt_n, mask_n = attention_ops.ragged_operands(k_one, vt_one, kv_len, q_len, mask, causal)
+            return self._mx_attend(q_mx, k_n, vt_n, mask_n, scaling, dtype)
         # The reference repeats K and V to the number of query heads and then quantizes (:189-213).  Every MX block lives inside
         # one head (K: along head_dim; V: along the sequence of one (head, channel) row), so quantizing the key/value heads once
         # and repeating the CODES is bit-identical -- a quarter of the quantization work and of the bytes copied under 4-way GQA.
@@ -394,11 +404,13 @@ class _MXAttentionMixin:
         key_states = k.view(hidden_shape).transpose(1, 2)
         value_states = v.view(hidden_shape).transpose(1, 2)
         cos, sin = position_embeddings
-        if isinstance(past_key_values, MXStaticCache) and self.qconfig.is_qkv_quantization_enabled:
+        if isinstance(past_key_values, (MXStaticCache, MXDynamicCache)) and self.qconfig.is_qkv_quantization_enabled:
             # the cache holds MX codes: rotary, the quantization of Q and the append of the new tokens' K / V blocks are one launch
-            # (K5e), and the attention reads the whole cache in place
-            q_mx, k_mx, vt_mx = past_key_values.layers[self.layer_idx].mx_append(query_states, key_states, value_states, cos, sin, self.qconfig)
-            attn_output = self._mx_attend(q_mx, k_mx, vt_mx, attention_mask, self.scaling, query_states.dtype)
+            # (K5e), and the attention reads the cache in place (a dynamic cache: its first `length` positions)
+            layer = past_key_values.layers[self.layer_idx]
+            q_mx, k_mx, vt_mx = layer.mx_append(query_states, key_states, value_states, cos, sin, self.qconfig)
+            kv_len = layer.length if isinstance(past_key_values, MXDynamicCache) else None
+            attn_output = self._mx_attend(q_mx, k_mx, vt_mx, attention_mask, self.scaling, query_states.dtype, kv_len=kv_len)
             return self.o_proj(attn_output.reshape(*input_shape, -1).contiguous()), None
         rotated = glue_ops.rope(query_states, key_states, cos, sin)  # one launch, the eager chain's roundings (K5b)
         query_states, key_states = rotated if rotated is not None else mod_llama.apply_rotary_pos_emb(query_states, key_states, cos, sin)
