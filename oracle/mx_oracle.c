@@ -12,8 +12,10 @@
  * MX_HARDWARE_EXACT_QUANTIZATION; the digests are committed in
  * tests/golden/digests.json and re-checked by tests/test_oracle_golden.py.
  * Exception: float8_e5m2 and fp32 input are not torchmx features at all
- * (torchmx/dtypes.py:143-149, torchmx/mx_tensor.py:59-61) -- for those two the
- * header of DESIGN.md says "parity unpinned".
+ * (torchmx/dtypes.py:143-149, torchmx/mx_tensor.py:59-61), so there is no
+ * reference output to pin them to.  The e5m2 path is pinned instead against a
+ * restatement built on torch's own float8_e5m2 cast (tests/test_e5m2_reference.py);
+ * fp32 input stays "parity unpinned" (header of DESIGN.md).
  *
  * Every function cites the reference lines (relative to /root/reference) it follows.
  * Plain C99, no dependencies beyond libm / pthreads.

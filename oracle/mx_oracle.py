@@ -26,7 +26,7 @@ ELEM_IDS = {
     "float6_e2m3": 2,
     "float4_e2m1": 3,
     "int8": 4,
-    "float8_e5m2": 5,  # extension, parity unpinned
+    "float8_e5m2": 5,  # extension: pinned against torch's float8_e5m2 cast (tests/test_e5m2_reference.py)
 }
 
 _lib = None
