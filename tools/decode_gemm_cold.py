@@ -14,7 +14,7 @@ for shape in os.environ.get("GT_SHAPES", "4096x4096,1024x4096,14336x4096,4096x14
     xb = torch.randn(M, K, device="cuda", dtype=torch.bfloat16)
     X = MXTensor.to_mx(xb, dtypes.float8_e4m3, 32)
     from torchmx_b200 import mx_gemm
-    run = (lambda W: mx_gemm.linear_fused_act_quant(xb, W, None, False)) if FUSED else (lambda W: torch.nn.functional.linear(X, W))
+    run = (lambda W: mx_gemm.linear_fused_act_quant(xb, W, None)) if FUSED else (lambda W: torch.nn.functional.linear(X, W))
     Ws = [MXTensor.to_mx(torch.randn(N, K, device="cuda", dtype=torch.bfloat16), wdt, 32) for _ in range(n_w)]
     for W in Ws:
         mx_gemm.mark_static(W)

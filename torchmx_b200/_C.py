@@ -205,5 +205,15 @@ def check(rc: int, what: str) -> None:
         raise RuntimeError(f"{what} failed (status {rc}): {lib().mxq_last_error().decode()}")
 
 
+def launch(name: str, *args) -> bool:
+    """`lib().<name>(*args)` for an entry the caller may decline: False when it refuses the shape (the caller then takes another
+    path), True when it ran.  Any other failure raises through `check`."""
+    rc = getattr(lib(), name)(*args)
+    if rc == ERR_UNSUPPORTED_SHAPE:
+        return False
+    check(rc, name)
+    return True
+
+
 def i64_array(values):
     return (ctypes.c_int64 * len(values))(*[int(v) for v in values])

@@ -14,8 +14,7 @@ from typing import Optional
 import torch
 
 from . import _C, dtypes
-from . import env_variables as env
-from .mx_tensor import MXTensor, _require_cuda, _stream_ptr
+from .mx_tensor import MXTensor, _codes_like, _quant_flags, _require_cuda, _stream_ptr
 
 stats = {"fused_softmax": 0, "unfused_softmax": 0, "flash_attention": 0}
 _ENABLED = os.environ.get("MXQ_FUSED_SOFTMAX", "1") != "0"
@@ -29,6 +28,21 @@ def set_fused_softmax(on: bool) -> bool:
     global _ENABLED
     prev, _ENABLED = _ENABLED, bool(on)
     return prev
+
+
+def _set_mask(a, mask: Optional[torch.Tensor], b: int, h: int, q_len: int, kv_len: int, device) -> bool:
+    """Point the mask fields of K4a's / K4b's arguments at `mask` (None, or additive bf16 on `device` broadcastable to
+    [b, h, q_len, >= kv_len] with kv stride 1); False when the mask does not qualify."""
+    if mask is None:
+        return True
+    if mask.dtype != torch.bfloat16 or mask.dim() != 4 or mask.device != device or mask.shape[-1] < kv_len or mask.shape[2] != q_len \
+            or mask.shape[0] not in (1, b) or mask.shape[1] not in (1, h) or (kv_len > 1 and mask.stride(3) != 1):
+        return False
+    a.mask = mask.data_ptr()
+    a.mask_stride_b = 0 if mask.shape[0] == 1 else mask.stride(0)
+    a.mask_stride_h = 0 if mask.shape[1] == 1 else mask.stride(1)
+    a.mask_stride_q = mask.stride(2)
+    return True
 
 
 def softmax_to_mx(scores: torch.Tensor, scaling: float, mask: Optional[torch.Tensor], causal: bool, elem_dtype: dtypes.DType,
@@ -45,29 +59,19 @@ def softmax_to_mx(scores: torch.Tensor, scaling: float, mask: Optional[torch.Ten
         return None
     _require_cuda(scores, "softmax_to_mx")
     a = _C.SoftmaxArgs()
-    if mask is not None:
-        if mask.dtype != torch.bfloat16 or mask.dim() != 4 or mask.device != scores.device or mask.shape[-1] < kv_len \
-                or mask.shape[2] != q_len or mask.shape[0] not in (1, b) or mask.shape[1] not in (1, h) or (kv_len > 1 and mask.stride(3) != 1):
-            return None
-        a.mask = mask.data_ptr()
-        a.mask_stride_b = 0 if mask.shape[0] == 1 else mask.stride(0)
-        a.mask_stride_h = 0 if mask.shape[1] == 1 else mask.stride(1)
-        a.mask_stride_q = mask.stride(2)
-    is_fp4 = elem_dtype == dtypes.float4_e2m1
-    codes = torch.empty((b, h, q_len, kv_len // 2 if is_fp4 else kv_len), dtype=torch.int8 if elem_dtype == dtypes.int8 else torch.uint8,
-                        device=scores.device)
+    if not _set_mask(a, mask, b, h, q_len, kv_len, scores.device):
+        return None
+    codes = _codes_like((b, h, q_len), kv_len, elem_dtype, scores.device)
     scales = torch.empty((b, h, q_len, kv_len // 32), dtype=torch.uint8, device=scores.device)
     a.scores = scores.data_ptr()
     a.batch, a.heads, a.q_len, a.kv_len = b, h, q_len, kv_len
     a.scaling = float(scaling)
     a.causal = 1 if causal else 0
     a.elem = dtypes.ELEM_ID[elem_dtype.name]
-    a.flags = _C.FLAG_HW_EXACT if (elem_dtype in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
+    a.flags = _quant_flags(elem_dtype)
     a.codes, a.scales = codes.data_ptr(), scales.data_ptr()
-    rc = _C.lib().mxq_softmax_quantize(a, scores.device.index, _stream_ptr(scores))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_softmax_quantize", a, scores.device.index, _stream_ptr(scores)):
         return None
-    _C.check(rc, "mxq_softmax_quantize")
     stats["fused_softmax"] += 1
     return MXTensor(scales, codes, elem_dtype, 32, scores.dtype)
 
@@ -139,14 +143,8 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
         return None
     dev = q_mx._data.device
     a = _C.AttentionArgs()
-    if mask is not None:
-        if mask.dtype != torch.bfloat16 or mask.dim() != 4 or mask.device != dev or mask.shape[-1] < kv_len or mask.shape[2] != q_len \
-                or mask.shape[0] not in (1, b) or mask.shape[1] not in (1, h) or (kv_len > 1 and mask.stride(3) != 1):
-            return None
-        a.mask = mask.data_ptr()
-        a.mask_stride_b = 0 if mask.shape[0] == 1 else mask.stride(0)
-        a.mask_stride_h = 0 if mask.shape[1] == 1 else mask.stride(1)
-        a.mask_stride_q = mask.stride(2)
+    if not _set_mask(a, mask, b, h, q_len, kv_len, dev):
+        return None
     (a.q_codes, a.q_format, a.q_scales), (a.k_codes, a.k_format, a.k_scales), (a.vt_codes, a.v_format, a.vt_scales) = \
         [(c.data_ptr(), f, s.data_ptr()) for c, f, s in ops]
     a.batch, a.heads, a.kv_heads, a.q_len, a.kv_len, a.head_dim = b, h, hk, q_len, kv_len, d
@@ -159,22 +157,19 @@ def flash_attention(q_mx: MXTensor, k_mx: MXTensor, vt_mx: MXTensor, scaling: fl
     if grouped:
         a.heads, a.q_len, a.mask_stride_q = hk, h // hk, 0
     a.p_elem = dtypes.ELEM_ID[p_elem_dtype.name]
-    a.flags = _C.FLAG_HW_EXACT if (p_elem_dtype in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
+    a.flags = _quant_flags(p_elem_dtype)
     out = torch.empty((b, q_len, h, d), dtype=torch.bfloat16, device=dev)
     a.out, a.out_batch_stride, a.out_row_stride, a.out_head_stride = out.data_ptr(), out.stride(0), out.stride(1), out.stride(2)
     if grouped:  # element (batch, key head, group row g, channel) of the kernel's view is head (key head * groups + g) of the one token
         a.out_row_stride, a.out_head_stride = out.stride(2), (h // hk) * out.stride(2)
     probs = None
     if return_probs:
-        is_fp4 = p_elem_dtype == dtypes.float4_e2m1
-        p_codes = torch.empty((b, h, q_len, n // 2 if is_fp4 else n), dtype=torch.uint8, device=dev)
+        p_codes = _codes_like((b, h, q_len), n, p_elem_dtype, dev)
         p_scales = torch.empty((b, h, q_len, n // 32), dtype=torch.uint8, device=dev)
         a.p_codes, a.p_scales = p_codes.data_ptr(), p_scales.data_ptr()
         probs = MXTensor(p_scales, p_codes, p_elem_dtype, 32, torch.bfloat16)
-    rc = _C.lib().mxq_flash_attention(a, dev.index, _stream_ptr(q_mx._data))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_flash_attention", a, dev.index, _stream_ptr(q_mx._data)):
         return None
-    _C.check(rc, "mxq_flash_attention")
     stats["flash_attention"] += 1
     return (out, probs) if return_probs else out
 

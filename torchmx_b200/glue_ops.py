@@ -20,9 +20,8 @@ from typing import Optional, Tuple
 import torch
 
 from . import _C, dtypes
-from . import env_variables as env
 from .mlp_ops import _rows_view
-from .mx_tensor import MXTensor, _stream_ptr
+from .mx_tensor import MXTensor, _codes_like, _quant_flags, _stream_ptr
 
 stats = {"rmsnorm": 0, "rmsnorm_to_mx": 0, "rope": 0, "quantize_heads": 0, "quantize_transposed": 0, "rope_quantize_kv": 0}
 _ENABLED = os.environ.get("MXQ_FUSED_GLUE", "1") != "0"
@@ -72,15 +71,12 @@ def rmsnorm(x: torch.Tensor, weight: torch.Tensor, eps: float, residual: Optiona
         a.y, a.ldy = y.data_ptr(), hidden
     if to_mx is not None:
         lead = tuple(x.shape[:-1])
-        is_fp4 = to_mx == dtypes.float4_e2m1
-        codes = torch.empty(lead + (hidden // 2 if is_fp4 else hidden,), dtype=torch.int8 if to_mx == dtypes.int8 else torch.uint8, device=x.device)
+        codes = _codes_like(lead, hidden, to_mx, x.device)
         scales = torch.empty(lead + (hidden // 32,), dtype=torch.uint8, device=x.device)
         a.codes, a.scales, a.elem = codes.data_ptr(), scales.data_ptr(), dtypes.ELEM_ID[to_mx.name]
-        a.flags = _C.FLAG_HW_EXACT if (to_mx in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
-    rc = _C.lib().mxq_rmsnorm(a, x.device.index, _stream_ptr(x))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+        a.flags = _quant_flags(to_mx)
+    if not _C.launch("mxq_rmsnorm", a, x.device.index, _stream_ptr(x)):
         return None
-    _C.check(rc, "mxq_rmsnorm")
     if to_mx is not None:
         mx = MXTensor(scales, codes, to_mx, 32, torch.bfloat16)
         stats["rmsnorm_to_mx"] += 1
@@ -104,6 +100,18 @@ def _out_view(t: torch.Tensor, like: torch.Tensor):
     return t.stride(0), t.stride(1), t.stride(2)
 
 
+def _set_rope_tables(a, cos: torch.Tensor, sin: torch.Tensor, b: int, t: int, d: int) -> bool:
+    """Point the cos / sin fields of K5b's / K5e's arguments at the tables ([b | 1, t, d], the same strides, unit last stride;
+    d > 1); False when they do not qualify."""
+    if cos.shape != sin.shape or cos.dim() != 3 or cos.shape[0] not in (1, b) or cos.shape[1] != t or cos.shape[2] != d \
+            or cos.stride() != sin.stride() or cos.stride(2) != 1:
+        return False
+    a.cos, a.sin = cos.data_ptr(), sin.data_ptr()
+    a.cs_tok_stride = cos.stride(1) if t > 1 else d
+    a.cs_batch_stride = cos.stride(0) if cos.shape[0] > 1 else 0
+    return True
+
+
 def rope(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor, k_out: Optional[torch.Tensor] = None,
          v: Optional[torch.Tensor] = None, v_out: Optional[torch.Tensor] = None) -> Optional[Tuple[torch.Tensor, torch.Tensor]]:
     """q / k: [batch, heads, tokens, head_dim] (transposed views of the [batch, tokens, heads * head_dim] projection outputs);
@@ -117,18 +125,16 @@ def rope(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor,
     if q.dim() != 4 or k.dim() != 4 or q.numel() == 0 or k.numel() == 0:
         return None
     b, hq, t, d = q.shape
-    if k.shape[0] != b or k.shape[2] != t or k.shape[3] != d or d % 16 or cos.shape != sin.shape or cos.dim() != 3 or cos.shape[0] not in (1, b) \
-            or cos.shape[1] != t or cos.shape[2] != d or cos.stride() != sin.stride() or (d > 1 and cos.stride(2) != 1):
+    if k.shape[0] != b or k.shape[2] != t or k.shape[3] != d or d % 16:
         return None
     qv, kv = _head_view(q, d), _head_view(k, d)
     if qv is None or kv is None:
         return None
     a = _C.RopeArgs()
+    if not _set_rope_tables(a, cos, sin, b, t, d):
+        return None
     a.q, a.q_batch_stride, a.q_tok_stride, a.q_heads = q.data_ptr(), qv[0], qv[1], hq
     a.k, a.k_batch_stride, a.k_tok_stride, a.k_heads = k.data_ptr(), kv[0], kv[1], k.shape[1]
-    a.cos, a.sin = cos.data_ptr(), sin.data_ptr()
-    a.cs_tok_stride = cos.stride(1) if t > 1 else d
-    a.cs_batch_stride = cos.stride(0) if cos.shape[0] > 1 else 0
     a.batch, a.tokens, a.head_dim = b, t, d
     q_out = torch.empty((b, hq, t, d), dtype=torch.bfloat16, device=q.device)
     if k_out is None:
@@ -148,10 +154,8 @@ def rope(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor,
         a.v_out = v_out.data_ptr()
         a.v_out_batch_stride, a.v_out_head_stride, a.v_out_tok_stride = vo
     a.q_out, a.k_out = q_out.data_ptr(), k_out.data_ptr()
-    rc = _C.lib().mxq_rope(a, q.device.index, _stream_ptr(q))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_rope", a, q.device.index, _stream_ptr(q)):
         return None
-    _C.check(rc, "mxq_rope")
     stats["rope"] += 1
     return q_out, k_out
 
@@ -165,15 +169,11 @@ def quantize_heads(x: torch.Tensor, elem_dtype: dtypes.DType, block_size: int = 
     b, h, t, d = x.shape
     if d % 32 or x.data_ptr() % 32:
         return None
-    is_fp4 = elem_dtype == dtypes.float4_e2m1
-    codes = torch.empty((b, t, h * d // 2 if is_fp4 else h * d), dtype=torch.int8 if elem_dtype == dtypes.int8 else torch.uint8, device=x.device)
+    codes = _codes_like((b, t), h * d, elem_dtype, x.device)
     scales = torch.empty((b, t, h * d // 32), dtype=torch.uint8, device=x.device)
-    flags = _C.FLAG_HW_EXACT if (elem_dtype in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
-    rc = _C.lib().mxq_quantize_heads(x.data_ptr(), b, h, t, d, dtypes.ELEM_ID[elem_dtype.name], flags, codes.data_ptr(), scales.data_ptr(),
-                                     x.device.index, _stream_ptr(x))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_quantize_heads", x.data_ptr(), b, h, t, d, dtypes.ELEM_ID[elem_dtype.name], _quant_flags(elem_dtype), codes.data_ptr(),
+                     scales.data_ptr(), x.device.index, _stream_ptr(x)):
         return None
-    _C.check(rc, "mxq_quantize_heads")
     stats["quantize_heads"] += 1
     return MXTensor(scales, codes, elem_dtype, 32, torch.bfloat16)
 
@@ -187,19 +187,16 @@ def quantize_transposed(x: torch.Tensor, elem_dtype: dtypes.DType, block_size: i
     n0, n1, rows, cols = x.shape
     if rows % 32 or cols % 8 or n0 * n1 > 65535 or x.data_ptr() % 16 or any(st % 8 for st in x.stride()[:3]):
         return None
-    is_fp4 = elem_dtype == dtypes.float4_e2m1
-    codes = torch.empty((n0, n1, cols, rows // 2 if is_fp4 else rows), dtype=torch.int8 if elem_dtype == dtypes.int8 else torch.uint8, device=x.device)
+    codes = _codes_like((n0, n1, cols), rows, elem_dtype, x.device)
     scales = torch.empty((n0, n1, cols, rows // 32), dtype=torch.uint8, device=x.device)
     a = _C.TransposedQuantArgs()
     a.x, a.n0, a.n1, a.rows, a.cols = x.data_ptr(), n0, n1, rows, cols
     a.s0, a.s1, a.row_stride = x.stride(0), x.stride(1), x.stride(2)
     a.elem = dtypes.ELEM_ID[elem_dtype.name]
-    a.flags = _C.FLAG_HW_EXACT if (elem_dtype in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
+    a.flags = _quant_flags(elem_dtype)
     a.codes, a.scales = codes.data_ptr(), scales.data_ptr()
-    rc = _C.lib().mxq_quantize_transposed(a, x.device.index, _stream_ptr(x))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_quantize_transposed", a, x.device.index, _stream_ptr(x)):
         return None
-    _C.check(rc, "mxq_quantize_transposed")
     stats["quantize_transposed"] += 1
     return MXTensor(scales, codes, elem_dtype, 32, torch.bfloat16)
 
@@ -227,8 +224,7 @@ def rope_quantize_kv(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, cos: tor
         return None
     b, hq, t, d = q.shape
     hk = k.shape[1]
-    if d != 128 or k.shape != (b, hk, t, d) or v.shape != k.shape or cos.shape != sin.shape or cos.dim() != 3 or cos.shape[0] not in (1, b) \
-            or cos.shape[1] != t or cos.shape[2] != d or cos.stride() != sin.stride() or cos.stride(2) != 1:
+    if d != 128 or k.shape != (b, hk, t, d) or v.shape != k.shape:
         return None
     qv, kv, vv = _head_view(q, d), _head_view(k, d), _head_view(v, d)
     if qv is None or kv is None or vv is None:
@@ -242,23 +238,20 @@ def rope_quantize_kv(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, cos: tor
     if position.dtype != torch.int64 or position.numel() != 1 or position.device != q.device:
         return None
     a = _C.RopeQuantizeKVArgs()
+    if not _set_rope_tables(a, cos, sin, b, t, d):
+        return None
     a.q, a.q_batch_stride, a.q_tok_stride, a.q_heads = q.data_ptr(), qv[0], qv[1], hq
     a.k, a.k_batch_stride, a.k_tok_stride = k.data_ptr(), kv[0], kv[1]
     a.v, a.v_batch_stride, a.v_tok_stride, a.kv_heads = v.data_ptr(), vv[0], vv[1], hk
-    a.cos, a.sin = cos.data_ptr(), sin.data_ptr()
-    a.cs_tok_stride = cos.stride(1) if t > 1 else d
-    a.cs_batch_stride = cos.stride(0) if cos.shape[0] > 1 else 0
     a.batch, a.tokens, a.head_dim = b, t, d
     a.q_elem, a.k_elem, a.v_elem = (dtypes.ELEM_ID[e.name] for e in elem_dtypes)
-    a.flags = _C.FLAG_HW_EXACT if env.MX_EXACT_QUANTIZATION == "True" else 0  # (e5m2 has no hardware-exact variant: the kernel ignores it there)
+    a.flags = _quant_flags(elem_dtypes[0]) | _quant_flags(elem_dtypes[1]) | _quant_flags(elem_dtypes[2])
     q_codes = torch.empty((b, hq, t, d), dtype=torch.uint8, device=q.device)
     q_scales = torch.empty((b, hq, t, d // 32), dtype=torch.uint8, device=q.device)
     a.q_codes, a.q_scales = q_codes.data_ptr(), q_scales.data_ptr()
     a.k_codes, a.k_scales, a.vt_codes, a.vt_scales = k_codes.data_ptr(), k_scales.data_ptr(), vt_codes.data_ptr(), vt_scales.data_ptr()
     a.v_open, a.capacity, a.position = v_open.data_ptr(), C, position.data_ptr()
-    rc = _C.lib().mxq_rope_quantize_kv(a, q.device.index, _stream_ptr(q))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_rope_quantize_kv", a, q.device.index, _stream_ptr(q)):
         return None
-    _C.check(rc, "mxq_rope_quantize_kv")
     stats["rope_quantize_kv"] += 1
     return MXTensor(q_scales, q_codes, byte_operand_dtype(elem_dtypes[0]), 32, torch.bfloat16)

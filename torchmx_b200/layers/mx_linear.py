@@ -9,7 +9,6 @@ from __future__ import annotations
 import torch
 import torch.nn.functional as F
 
-from .. import env_variables as env
 from .. import mx_gemm
 from ..config import QLinearConfig
 from ..mx_tensor import MXTensor
@@ -92,12 +91,12 @@ class MXInferenceLinear(torch.nn.Linear):
         w_mx = self._weight_mx()
         if ac.elem_dtype_name == "float8_e4m3" and ac.block_size == 32:
             # decode-sized activations: quantization fused into the weight-streaming GEMM (one launch, no code round trip)
-            out = mx_gemm.linear_fused_act_quant(x, w_mx, bias, env.MX_EXACT_QUANTIZATION == "True", fused=_fused)
+            out = mx_gemm.linear_fused_act_quant(x, w_mx, bias, fused=_fused)
             if out is not None:
                 return out
         elif ac.block_size == 32 and ac.elem_dtype_name in ("float6_e3m2", "float6_e2m3", "float4_e2m1"):
             # 4 / 6-bit activations: K1 writes the packed operand stream the GEMM reads (no mxq_pack_operand launch in between)
-            out = mx_gemm.linear_packed_act_quant(x, w_mx, bias, ac.elem_dtype, env.MX_EXACT_QUANTIZATION == "True", fused=_fused)
+            out = mx_gemm.linear_packed_act_quant(x, w_mx, bias, ac.elem_dtype, fused=_fused)
             if out is not None:
                 return out
         x_mx = MXTensor.to_mx(x, ac.elem_dtype, ac.block_size)

@@ -105,7 +105,7 @@ def _stacked_from_float(srcs, qconfig: QLinearConfig):
     scales: no per-projection tensors, no concatenation (and, across the layers of a model, the stacked gate/up codes are exactly
     the size of a bf16 projection weight being released, so the caching allocator serves them without going to the driver).  Same
     kernel per projection, same bytes.  None when the modules do not qualify (the caller converts them one by one)."""
-    from ..mx_tensor import _empty_scales, _quantize_into
+    from ..mx_tensor import _codes_like, _empty_scales, _quantize_into
     wc = qconfig.weights_config
     ws = [getattr(m, "weight", None) for m in srcs]
     w0 = ws[0]
@@ -118,7 +118,7 @@ def _stacked_from_float(srcs, qconfig: QLinearConfig):
     if srcs[0].bias is not None and any(m.bias.dtype != torch.bfloat16 or m.bias.device != w0.device for m in srcs):
         return None
     rows = [w.shape[0] for w in ws]
-    codes = torch.empty((sum(rows), K // 2 if elem.name == "float4_e2m1" else K), dtype=torch.int8 if elem.name == "int8" else torch.uint8, device=w0.device)
+    codes = _codes_like((sum(rows),), K, elem, w0.device)
     scales = _empty_scales((sum(rows), K // bs), w0.device)
     layers, row = [], 0
     bias_all = torch.cat([m.bias.data for m in srcs], 0) if srcs[0].bias is not None else None

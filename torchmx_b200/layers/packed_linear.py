@@ -14,7 +14,6 @@ from __future__ import annotations
 import torch
 
 from .. import dtypes, mx_gemm
-from .. import env_variables as env
 from ..config import QLinearConfig
 from ..mx_tensor import MXTensor
 from .mx_linear import MXInferenceLinear
@@ -108,5 +107,4 @@ class PackedMXLinear(torch.nn.Module):
             "a packed-only weight needs an FP activation format with block size 32 (no dequantize fallback)"
         if isinstance(x, MXTensor):
             assert x._elem_dtype == ac.elem_dtype and x._block_size == ac.block_size, "activation was quantized with another config"
-        return mx_gemm.linear_packed_weight(x, self.weight_packed, self.weight_scale, self.operand_format, self.bias, ac.elem_dtype,
-                                            env.MX_EXACT_QUANTIZATION == "True", owner=self)
+        return mx_gemm.linear_packed_weight(x, self.weight_packed, self.weight_scale, self.operand_format, self.bias, ac.elem_dtype, owner=self)

@@ -12,8 +12,7 @@ from typing import Optional
 import torch
 
 from . import _C, dtypes
-from . import env_variables as env
-from .mx_tensor import MXTensor, _stream_ptr
+from .mx_tensor import MXTensor, _codes_like, _quant_flags, _stream_ptr
 
 stats = {"fused_silu_mul": 0}
 _ENABLED = os.environ.get("MXQ_FUSED_SILU_MUL", "1") != "0"
@@ -56,14 +55,10 @@ def silu_mul_to_mx(gate: torch.Tensor, up: torch.Tensor, elem_dtype: dtypes.DTyp
         return None
     rows = gate.numel() // cols
     lead = tuple(gate.shape[:-1])
-    is_fp4 = elem_dtype == dtypes.float4_e2m1
-    codes = torch.empty(lead + (cols // 2 if is_fp4 else cols,), dtype=torch.int8 if elem_dtype == dtypes.int8 else torch.uint8, device=gate.device)
+    codes = _codes_like(lead, cols, elem_dtype, gate.device)
     scales = torch.empty(lead + (cols // 32,), dtype=torch.uint8, device=gate.device)
-    flags = _C.FLAG_HW_EXACT if (elem_dtype in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
-    rc = _C.lib().mxq_silu_mul_quantize(gate.data_ptr(), up.data_ptr(), rows, cols, ldg, ldu, dtypes.ELEM_ID[elem_dtype.name], flags,
-                                        codes.data_ptr(), scales.data_ptr(), gate.device.index, _stream_ptr(gate))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_silu_mul_quantize", gate.data_ptr(), up.data_ptr(), rows, cols, ldg, ldu, dtypes.ELEM_ID[elem_dtype.name],
+                     _quant_flags(elem_dtype), codes.data_ptr(), scales.data_ptr(), gate.device.index, _stream_ptr(gate)):
         return None
-    _C.check(rc, "mxq_silu_mul_quantize")
     stats["fused_silu_mul"] += 1
     return MXTensor(scales, codes, elem_dtype, 32, gate.dtype)

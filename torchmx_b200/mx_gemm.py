@@ -16,7 +16,7 @@ from typing import Optional
 import torch
 
 from . import _C, dtypes
-from .mx_tensor import MXTensor, _stream_ptr
+from .mx_tensor import MXTensor, _codes_like, _quant_flags, _stream_ptr
 
 aten = torch.ops.aten
 
@@ -26,8 +26,11 @@ _SHADOW_ATTR = "_mxq_e4m3_shadow"
 
 # tensor_core: launches of the block-scaled tcgen05 kernels (K3a/b/c); dequant_gemm: launches of the fused dequantize + bf16
 # tcgen05 kernel (K3d) for operands the block-scaled instruction cannot take; fallback: contractions that reached neither and
-# ran as K2 + aten (torch.compile tracing, non-bf16 advertised dtypes)
-stats = {"tensor_core": 0, "dequant_gemm": 0, "fallback": 0, "transcode": 0, "fused_allreduce": 0}
+# ran as K2 + aten (torch.compile tracing, non-bf16 advertised dtypes); dequant_once_gemm: the dequant_gemm launches that
+# dequantized each operand once first; fused_act_quant / packed_act_quant: the tensor_core launches whose bf16 activation was
+# quantized inside the GEMM / written by K1 as the packed operand stream
+stats = {"tensor_core": 0, "dequant_gemm": 0, "dequant_once_gemm": 0, "fallback": 0, "transcode": 0, "fused_allreduce": 0,
+         "fused_act_quant": 0, "packed_act_quant": 0}
 
 class FusedOutput:
     """Target of a fused GEMM + all-reduce launch, handed EXPLICITLY from RowParallelMXLinear.forward down to the launch (no
@@ -169,11 +172,7 @@ def _launch(a_codes, sfa, b_codes, sfb, bias, batch, M, N, K, a_bs, sfa_bs, b_bs
     g.bias = bias.data_ptr() if bias is not None else None
     g.d, g.ldd, g.d_batch_stride = out.data_ptr(), N, M * N
     g.batch, g.M, g.N, g.K = batch, M, N, K
-    rc = _C.lib().mxq_gemm(ctypes.byref(g), out.device.index, _stream_ptr(out))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
-        return False
-    _C.check(rc, "mxq_gemm")
-    return True
+    return _C.launch("mxq_gemm", ctypes.byref(g), out.device.index, _stream_ptr(out))
 
 
 def try_tensor_core(aten_op, a: MXTensor, b: MXTensor, extra_front, extra_back, count_fallback: bool = True,
@@ -289,12 +288,10 @@ def try_dequant_gemm(aten_op, a: MXTensor, b: MXTensor, extra_front, extra_back)
         a_hp = a.to_dtype(torch.bfloat16).reshape(batch, M, K)
         b_hp = (b if b_k == -1 else b.transpose(-1, -2)).to_dtype(torch.bfloat16).reshape(batch, N, K)
         out = torch.empty(lead + (N,), dtype=torch.bfloat16, device=a._data.device)
-        rc = _C.lib().mxq_gemm_bf16(a_hp.data_ptr(), K, M * K, b_hp.data_ptr(), K, N * K, bias.data_ptr() if bias is not None else None, out.data_ptr(), N, M * N,
-                                    batch, M, N, K, out.device.index, _stream_ptr(out))
-        if rc != _C.ERR_UNSUPPORTED_SHAPE:
-            _C.check(rc, "mxq_gemm_bf16")
+        if _C.launch("mxq_gemm_bf16", a_hp.data_ptr(), K, M * K, b_hp.data_ptr(), K, N * K, bias.data_ptr() if bias is not None else None,
+                     out.data_ptr(), N, M * N, batch, M, N, K, out.device.index, _stream_ptr(out)):
             stats["dequant_gemm"] += 1
-            stats["dequant_once_gemm"] = stats.get("dequant_once_gemm", 0) + 1
+            stats["dequant_once_gemm"] += 1
             return out
     g = _C.GemmDequantArgs()
     keep_a = _fill_operand(g.a, a, -2, -1, batched, collapse=aten_op is aten.linear.default)
@@ -309,10 +306,8 @@ def try_dequant_gemm(aten_op, a: MXTensor, b: MXTensor, extra_front, extra_back)
     g.bias = bias.data_ptr() if bias is not None else None
     g.d, g.ldd, g.d_batch_stride = out.data_ptr(), N, M * N
     g.batch, g.M, g.N, g.K = batch, M, N, K
-    rc = _C.lib().mxq_gemm_dequant(ctypes.byref(g), out.device.index, _stream_ptr(out))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_gemm_dequant", ctypes.byref(g), out.device.index, _stream_ptr(out)):
         return None
-    _C.check(rc, "mxq_gemm_dequant")
     del keep_a, keep_b
     stats["dequant_gemm"] += 1
     return out
@@ -412,7 +407,7 @@ _FUSED_ACT = os.environ.get("MXQ_FUSED_ACT_QUANT", "1") != "0"
 FUSED_ACT_MAX_ROWS = 64
 
 
-def linear_fused_act_quant(x: torch.Tensor, w: MXTensor, bias, hw_exact: bool, fused: Optional[FusedOutput] = None) -> Optional[torch.Tensor]:
+def linear_fused_act_quant(x: torch.Tensor, w: MXTensor, bias, fused: Optional[FusedOutput] = None) -> Optional[torch.Tensor]:
     """MXInferenceLinear.forward for decode-sized activations in ONE launch: y = quantize_mx(x, float8_e4m3, 32) @ w^T (+ bias)
     with the quantization done inside the weight-streaming kernel (bit-identical to the two-launch path).  Returns None when
     the operands do not qualify; the caller then quantizes with K1 and goes through `try_tensor_core`."""
@@ -439,11 +434,11 @@ def linear_fused_act_quant(x: torch.Tensor, w: MXTensor, bias, hw_exact: bool, f
         fused, d_mc = None, 0
         out = torch.empty(tuple(x.shape[:-1]) + (N,), dtype=torch.bfloat16, device=x.device)
     ok = _launch(None, None, b_e, wk[1], bias, 1, rows, N, K, 0, 0, 0, 0, out, FMT_E4M3_BYTES, b_fmt, d_mc, x_hp=x2,
-                 x_flags=_C.FLAG_HW_EXACT if hw_exact else 0, static_b=_static_b(w_origin))
+                 x_flags=_quant_flags(dtypes.float8_e4m3), static_b=_static_b(w_origin))
     if not ok:
         return None
     stats["tensor_core"] += 1
-    stats["fused_act_quant"] = stats.get("fused_act_quant", 0) + 1
+    stats["fused_act_quant"] += 1
     if fused is not None:
         fused.taken = True
         stats["fused_allreduce"] += 1
@@ -451,7 +446,7 @@ def linear_fused_act_quant(x: torch.Tensor, w: MXTensor, bias, hw_exact: bool, f
     return out
 
 
-def linear_packed_act_quant(x: torch.Tensor, w: MXTensor, bias, act_elem: dtypes.DType, hw_exact: bool,
+def linear_packed_act_quant(x: torch.Tensor, w: MXTensor, bias, act_elem: dtypes.DType,
                             fused: Optional[FusedOutput] = None) -> Optional[torch.Tensor]:
     """MXInferenceLinear.forward with a 4 / 6-bit ACTIVATION config (reference: torchmx/layers/mx_linear.py:63-94 with
     `activations_config` float6_* / float4_e2m1): K1 writes the packed tensor-core operand stream itself (MXQ_FLAG_OPERAND_LAYOUT)
@@ -475,11 +470,9 @@ def linear_packed_act_quant(x: torch.Tensor, w: MXTensor, bias, act_elem: dtypes
     a_fmt = _PACKED_FORMAT[act_elem.name]
     a_e = torch.empty((rows, K * _PACKED_BITS[a_fmt] // 8), dtype=torch.uint8, device=x.device)
     sfa = torch.empty((rows, K // 32), dtype=torch.uint8, device=x.device)
-    rc = _C.lib().mxq_quantize(x.data_ptr(), _C.HP_BF16, rows * (K // 32), 32, dtypes.ELEM_ID[act_elem.name],
-                               _C.FLAG_OPERAND_LAYOUT | (_C.FLAG_HW_EXACT if hw_exact else 0), a_e.data_ptr(), sfa.data_ptr(), x.device.index, _stream_ptr(x))
-    if rc == _C.ERR_UNSUPPORTED_SHAPE:
+    if not _C.launch("mxq_quantize", x.data_ptr(), _C.HP_BF16, rows * (K // 32), 32, dtypes.ELEM_ID[act_elem.name],
+                     _C.FLAG_OPERAND_LAYOUT | _quant_flags(act_elem), a_e.data_ptr(), sfa.data_ptr(), x.device.index, _stream_ptr(x)):
         return None
-    _C.check(rc, "mxq_quantize")
     w_origin = getattr(w, "_mxq_origin", w)
     b_e, b_fmt = _operand_rows(wk[0], w._elem_dtype, w_origin)
     N = w.shape[0]
@@ -496,7 +489,7 @@ def linear_packed_act_quant(x: torch.Tensor, w: MXTensor, bias, act_elem: dtypes
     if not ok:
         return None
     stats["tensor_core"] += 1
-    stats["packed_act_quant"] = stats.get("packed_act_quant", 0) + 1
+    stats["packed_act_quant"] += 1
     if fused is not None:
         fused.taken = True
         stats["fused_allreduce"] += 1
@@ -519,14 +512,14 @@ def unpack_weight(packed: torch.Tensor, fmt: int, elem: dtypes.DType) -> torch.T
         return packed.clone()
     bits = _PACKED_BITS[fmt]
     k = packed.shape[-1] * 8 // bits
-    out = torch.empty(tuple(packed.shape[:-1]) + (k // 2 if elem == dtypes.float4_e2m1 else k,), dtype=torch.uint8, device=packed.device)
+    out = _codes_like(packed.shape[:-1], k, elem, packed.device)
     rc = _C.lib().mxq_unpack_operand(packed.data_ptr(), dtypes.ELEM_ID[elem.name], packed.numel() * 8 // bits, out.data_ptr(),
                                      packed.device.index, _stream_ptr(packed))
     _C.check(rc, "mxq_unpack_operand")
     return out
 
 
-def linear_packed_weight(x, b_e: torch.Tensor, sfb: torch.Tensor, b_fmt: int, bias, act_elem: dtypes.DType, hw_exact: bool, owner=None) -> torch.Tensor:
+def linear_packed_weight(x, b_e: torch.Tensor, sfb: torch.Tensor, b_fmt: int, bias, act_elem: dtypes.DType, owner=None) -> torch.Tensor:
     """y = quantize_mx(x, act_elem, 32) @ W^T (+ bias) for a weight held only as its tensor-core operand (`pack_weight`).
     x: bf16 [..., K] or an MXTensor already quantized with the layer's activation config.  Decode-sized bf16 activations
     are quantized inside the GEMM; everything else goes K1 -> K3.  Raises if the launch is refused: there is no other path."""
@@ -543,10 +536,10 @@ def linear_packed_weight(x, b_e: torch.Tensor, sfb: torch.Tensor, b_fmt: int, bi
     if (not isinstance(x, MXTensor) and _FUSED_ACT and act_elem == dtypes.float8_e4m3 and rows <= FUSED_ACT_MAX_ROWS and x.is_contiguous()
             and x.dtype == torch.bfloat16):
         ok = _launch(None, None, b_e, sfb, bias, 1, rows, N, K, 0, 0, 0, 0, out, FMT_E4M3_BYTES, b_fmt, 0, x_hp=x.view(rows, K),
-                     x_flags=_C.FLAG_HW_EXACT if hw_exact else 0, static_b=static_b)
+                     x_flags=_quant_flags(act_elem), static_b=static_b)
         if ok:
             stats["tensor_core"] += 1
-            stats["fused_act_quant"] = stats.get("fused_act_quant", 0) + 1
+            stats["fused_act_quant"] += 1
             return out
     if (not isinstance(x, MXTensor) and _USE_PACKED and act_elem.name in _PACKED_FORMAT and type(x) is torch.Tensor and x.dtype == torch.bfloat16
             and x.is_contiguous() and x.data_ptr() % 32 == 0):
@@ -554,11 +547,11 @@ def linear_packed_weight(x, b_e: torch.Tensor, sfb: torch.Tensor, b_fmt: int, bi
         a_fmt = _PACKED_FORMAT[act_elem.name]
         a_e = torch.empty((rows, K * _PACKED_BITS[a_fmt] // 8), dtype=torch.uint8, device=x.device)
         sfa = torch.empty((rows, K // 32), dtype=torch.uint8, device=x.device)
-        rc = _C.lib().mxq_quantize(x.data_ptr(), _C.HP_BF16, rows * (K // 32), 32, dtypes.ELEM_ID[act_elem.name],
-                                   _C.FLAG_OPERAND_LAYOUT | (_C.FLAG_HW_EXACT if hw_exact else 0), a_e.data_ptr(), sfa.data_ptr(), x.device.index, _stream_ptr(x))
-        if rc == _C.OK and _launch(a_e, sfa, b_e, sfb, bias, 1, rows, N, K, 0, 0, 0, 0, out, a_fmt, b_fmt, 0, static_b=static_b):
+        if (_C.launch("mxq_quantize", x.data_ptr(), _C.HP_BF16, rows * (K // 32), 32, dtypes.ELEM_ID[act_elem.name],
+                      _C.FLAG_OPERAND_LAYOUT | _quant_flags(act_elem), a_e.data_ptr(), sfa.data_ptr(), x.device.index, _stream_ptr(x))
+                and _launch(a_e, sfa, b_e, sfb, bias, 1, rows, N, K, 0, 0, 0, 0, out, a_fmt, b_fmt, 0, static_b=static_b)):
             stats["tensor_core"] += 1
-            stats["packed_act_quant"] = stats.get("packed_act_quant", 0) + 1
+            stats["packed_act_quant"] += 1
             return out
     x_mx = x if isinstance(x, MXTensor) else MXTensor.to_mx(x, act_elem, 32)
     assert _qualifies(x_mx) and x_mx._block_dim == x_mx._data.dim() - 1 and x_mx._data.is_contiguous(), "activation cannot run on the tensor-core path"

@@ -42,6 +42,23 @@ def _stream_ptr(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
 
 
+def _quant_flags(elem: dtypes.DType) -> int:
+    """MXQ_FLAG_HW_EXACT when the reference's hardware-exact quantization is on and `elem` is one of the four element types it
+    applies to (mx_tensor.py:80-90), else 0.  `env` is read at call time: callers may flip it after import."""
+    return _C.FLAG_HW_EXACT if env.MX_EXACT_QUANTIZATION == "True" and elem in dtypes.SUPPORTED_FP_ELEM_DTYPES else 0
+
+
+def _codes_shape(lead, cols, elem: dtypes.DType) -> Tuple[tuple, torch.dtype]:
+    """(shape, dtype) of the codes of `cols` elements per row, blocked along the last axis: fp4 packs two codes per byte, int8
+    codes are int8, every other element type is one uint8 per element"""
+    return tuple(lead) + (cols // 2 if elem == dtypes.float4_e2m1 else cols,), torch.int8 if elem == dtypes.int8 else torch.uint8
+
+
+def _codes_like(lead, cols, elem: dtypes.DType, device) -> torch.Tensor:
+    shape, dtype = _codes_shape(lead, cols, elem)
+    return torch.empty(shape, dtype=dtype, device=device)
+
+
 # ------------------------------------------------------------------------------------------------
 # where the scale tensors of a whole-model quantization live
 # ------------------------------------------------------------------------------------------------
@@ -98,16 +115,10 @@ def _quantize_mx_impl(data_hp: torch.Tensor, elem_dtype_name: str, block_size: i
     shape = tuple(x.shape)
     n_blocks = x.numel() // block_size
     scales = _empty_scales(shape[:-1] + (shape[-1] // block_size,), x.device)
-    if elem == dtypes.float4_e2m1:
-        assert shape[-1] % 2 == 0  # pack_uint4's requirement (utils.py:143)
-        codes = torch.empty(shape[:-1] + (shape[-1] // 2,), dtype=torch.uint8, device=x.device)
-    else:
-        codes = torch.empty(shape, dtype=torch.int8 if elem == dtypes.int8 else torch.uint8, device=x.device)
-    flags = 0
-    if elem in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True":
-        flags |= _C.FLAG_HW_EXACT  # mx_tensor.py:80-90
+    assert elem != dtypes.float4_e2m1 or shape[-1] % 2 == 0  # pack_uint4's requirement (utils.py:143)
+    codes = _codes_like(shape[:-1], shape[-1], elem, x.device)
     if n_blocks:
-        rc = _C.lib().mxq_quantize(x.data_ptr(), _HP_ID[x.dtype], n_blocks, block_size, dtypes.ELEM_ID[elem.name], flags,
+        rc = _C.lib().mxq_quantize(x.data_ptr(), _HP_ID[x.dtype], n_blocks, block_size, dtypes.ELEM_ID[elem.name], _quant_flags(elem),
                                    codes.data_ptr(), scales.data_ptr(), x.device.index, _stream_ptr(x))
         _C.check(rc, "torchmx::quantize_mx")
     return scales, codes
@@ -120,10 +131,9 @@ def _quantize_into(data_hp: torch.Tensor, elem: dtypes.DType, block_size: int, c
     assert data_hp.shape[-1] % block_size == 0 and scales_out.numel() * block_size == data_hp.numel()
     assert codes_out.numel() * (2 if elem == dtypes.float4_e2m1 else 1) == data_hp.numel() and codes_out.device == data_hp.device == scales_out.device
     _require_cuda(data_hp, "torchmx::quantize_mx")
-    flags = _C.FLAG_HW_EXACT if (elem in dtypes.SUPPORTED_FP_ELEM_DTYPES and env.MX_EXACT_QUANTIZATION == "True") else 0
     if data_hp.numel():
-        rc = _C.lib().mxq_quantize(data_hp.data_ptr(), _HP_ID[data_hp.dtype], data_hp.numel() // block_size, block_size, dtypes.ELEM_ID[elem.name], flags,
-                                   codes_out.data_ptr(), scales_out.data_ptr(), data_hp.device.index, _stream_ptr(data_hp))
+        rc = _C.lib().mxq_quantize(data_hp.data_ptr(), _HP_ID[data_hp.dtype], data_hp.numel() // block_size, block_size, dtypes.ELEM_ID[elem.name],
+                                   _quant_flags(elem), codes_out.data_ptr(), scales_out.data_ptr(), data_hp.device.index, _stream_ptr(data_hp))
         _C.check(rc, "torchmx::quantize_mx")
 
 
@@ -135,14 +145,10 @@ def quantize_mx(data_hp: torch.Tensor, elem_dtype_name: str, block_size: int) ->
 
 @quantize_mx.register_fake
 def _(data_hp: torch.Tensor, elem_dtype_name: str, block_size: int) -> Tuple[torch.Tensor, torch.Tensor]:
-    elem = dtypes.STR_TO_ELEM_DTYPE[elem_dtype_name]
     shape = tuple(data_hp.shape)
     scales = data_hp.new_empty(shape[:-1] + (shape[-1] // block_size,), dtype=torch.uint8)
-    if elem == dtypes.float4_e2m1:
-        codes = data_hp.new_empty(shape[:-1] + (shape[-1] // 2,), dtype=torch.uint8)
-    else:
-        codes = data_hp.new_empty(shape, dtype=torch.int8 if elem == dtypes.int8 else torch.uint8)
-    return scales, codes
+    codes_shape, codes_dtype = _codes_shape(shape[:-1], shape[-1], dtypes.STR_TO_ELEM_DTYPE[elem_dtype_name])
+    return scales, data_hp.new_empty(codes_shape, dtype=codes_dtype)
 
 
 def _collapse_around(t_sizes, t_strides, d):
