@@ -431,13 +431,76 @@ typedef struct {
 } mxq_rope_quantize_kv_args_t;
 MXQ_API int mxq_rope_quantize_kv(const mxq_rope_quantize_kv_args_t *args, int device, void *stream);
 
+/*
+ * Mixture-of-experts layer (K6)  <->  transformers' expert loop over a fused expert bank (MixtralExperts.forward and its Qwen2-MoE /
+ * Qwen3-MoE / OLMoE twins: gate_up_proj [E, 2I, H], down_proj [E, H, I], SiLU gating) with every F.linear an MX matmul.  Three
+ * entries; none reads a device value on the host, so a step built from them can be captured in a CUDA graph.
+ *
+ * mxq_moe_route: top_k_index [tokens, top_k] int64 -> a stable counting sort of the (token, slot) pairs by expert.  Slots whose
+ * expert is outside [0, num_experts) are dropped (the loop skips them too).
+ *   offsets      : int32 [num_experts + 1]: the routed rows of expert e are offsets[e] .. offsets[e + 1] - 1, ordered by
+ *                  (token, slot); offsets[num_experts] = number of routed rows R <= tokens * top_k
+ *   row_of_slot  : int32 [tokens * top_k]: routed row of (t, s) at t * top_k + s, -1 for a dropped slot
+ *   token_of_row : int32 [tokens * top_k]: token of each routed row (entries >= R are not written)
+ *   x / codes / scales : optional (all NULL or none): x bf16 [tokens, hidden] (row stride ldx elements, a multiple of 8, 16-byte
+ *                  aligned base); routed row r of codes [tokens * top_k, hidden] (hidden / 2 bytes for MXQ_ELEM_E2M1) and scales
+ *                  [tokens * top_k, hidden / 32] receives quantize_mx(x[token_of_row[r]], elem, 32) (mxq_quantize's arithmetic)
+ * MXQ_ERR_INVALID: a NULL pointer, top_k outside 1..8, num_experts outside 1..256, tokens outside 0..16384, an unknown element type;
+ * MXQ_ERR_UNSUPPORTED_SHAPE: hidden % 32 != 0 or a misaligned x / codes (16 bytes) when quantizing.
+ */
+#define MXQ_MOE_MAX_EXPERTS 256
+#define MXQ_MOE_MAX_TOP_K 8
+#define MXQ_MOE_MAX_TOKENS 16384
+typedef struct {
+    const int64_t *top_k_index; int64_t tokens; int top_k; int num_experts;
+    int32_t *offsets; int32_t *row_of_slot; int32_t *token_of_row;
+    const void *x; int64_t ldx; int64_t hidden;
+    int elem /* mxq_elem_t */; unsigned flags /* MXQ_FLAG_HW_EXACT */;
+    void *codes; uint8_t *scales;
+} mxq_moe_route_args_t;
+MXQ_API int mxq_moe_route(const mxq_moe_route_args_t *args, int device, void *stream);
+
+/*
+ * mxq_moe_gemm: D[r, :] = X[r, :] . W[e(r)]^T for every routed row r < offsets[num_experts], where e(r) is the expert whose
+ * segment holds r -- one launch for all experts, the offsets read on the device.  Experts without rows cost no weight bytes.
+ *   w_codes  : [num_experts * N, K] in operand format w_format (MXQ_OPERAND_*), rows compact (K * bits / 8 bytes);
+ *   w_scales : [num_experts * N, K / 32] E8M0
+ *   x_codes  : [rows, K] in x_format, compact rows; x_scales [rows, K / 32]; rows = the capacity the offsets index into
+ *   d        : bf16 [rows, N]; only rows < offsets[num_experts] are written
+ * MXQ_ERR_INVALID: a NULL pointer, num_experts outside 1..256, an unknown operand format;
+ * MXQ_ERR_UNSUPPORTED_SHAPE: K % 128 != 0, N % 128 != 0, code pointers not 32-byte aligned, d or scales not 16-byte aligned.
+ */
+typedef struct {
+    const void *w_codes; const uint8_t *w_scales; int w_format;
+    const void *x_codes; const uint8_t *x_scales; int x_format;
+    const int32_t *offsets;
+    void *d;
+    int64_t rows, num_experts, N, K;
+} mxq_moe_gemm_args_t;
+MXQ_API int mxq_moe_gemm(const mxq_moe_gemm_args_t *args, int device, void *stream);
+
+/*
+ * mxq_moe_combine: out[t, :] = the loop's successive index_add_ calls: starting from +0, for the token's slots in ascending
+ * expert order, out = bf16(out + bf16(fp32(y[row_of_slot[t, s], :]) * w[t, s])).  One write per output element, no atomics.
+ *   y : bf16 [*, hidden] routed rows (mxq_moe_gemm's D), top_k_index / row_of_slot as mxq_moe_route's,
+ *   top_k_weights : [tokens, top_k] of weights_dtype (MXQ_HP_F32 or MXQ_HP_BF16), out : bf16 [tokens, hidden]
+ * MXQ_ERR_INVALID as mxq_moe_route; MXQ_ERR_UNSUPPORTED_SHAPE: hidden % 8 != 0, y / out not 16-byte aligned.
+ */
+typedef struct {
+    const void *y; const int64_t *top_k_index; const void *top_k_weights; int weights_dtype /* mxq_hp_t */;
+    const int32_t *row_of_slot;
+    int64_t tokens; int top_k; int num_experts; int64_t hidden;
+    void *out;
+} mxq_moe_combine_args_t;
+MXQ_API int mxq_moe_combine(const mxq_moe_combine_args_t *args, int device, void *stream);
+
 #define MXQ_OK 0
 #define MXQ_ERR_INVALID 1
 #define MXQ_ERR_UNSUPPORTED_SHAPE 2
 #define MXQ_ERR_CUDA 3
 
 MXQ_API const char *mxq_last_error(void);
-/* ABI version: 5 (mxq_attention_args_t.kv_pitch) */
+/* ABI version: 6 (the mxq_moe_* entries) */
 MXQ_API int mxq_version(void);
 /* compiled-for architecture as an integer (1000 for sm_100a) -- lets the host refuse to run a
  * library that was built for something else instead of failing inside a launch. */

@@ -14,12 +14,12 @@ HP_BF16, HP_F32 = 0, 1
 FLAG_HW_EXACT = 1
 FLAG_OPERAND_LAYOUT = 2
 GEMM_B_STATIC, GEMM_WIDE_TILES, GEMM_NO_PDL, GEMM_NO_MXF4 = 1, 2, 4, 8
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_DIMS = 6
 
 EXPORTS = ("mxq_quantize", "mxq_dequantize", "mxq_dequantize_strided", "mxq_gemm", "mxq_gemm_dequant", "mxq_gemm_bf16", "mxq_transcode_to_e4m3", "mxq_pack_operand", "mxq_unpack_operand",
            "mxq_softmax_quantize", "mxq_flash_attention", "mxq_silu_mul_quantize", "mxq_rmsnorm", "mxq_rope", "mxq_quantize_heads", "mxq_quantize_transposed", "mxq_rope_quantize_kv",
-           "mxq_last_error", "mxq_version", "mxq_arch")
+           "mxq_moe_route", "mxq_moe_gemm", "mxq_moe_combine", "mxq_last_error", "mxq_version", "mxq_arch")
 
 
 class GemmArgs(ctypes.Structure):
@@ -136,6 +136,35 @@ class RopeQuantizeKVArgs(ctypes.Structure):
     ]
 
 
+class MoeRouteArgs(ctypes.Structure):
+    _fields_ = [
+        ("top_k_index", ctypes.c_void_p), ("tokens", ctypes.c_int64), ("top_k", ctypes.c_int), ("num_experts", ctypes.c_int),
+        ("offsets", ctypes.c_void_p), ("row_of_slot", ctypes.c_void_p), ("token_of_row", ctypes.c_void_p),
+        ("x", ctypes.c_void_p), ("ldx", ctypes.c_int64), ("hidden", ctypes.c_int64),
+        ("elem", ctypes.c_int), ("flags", ctypes.c_uint),
+        ("codes", ctypes.c_void_p), ("scales", ctypes.c_void_p),
+    ]
+
+
+class MoeGemmArgs(ctypes.Structure):
+    _fields_ = [
+        ("w_codes", ctypes.c_void_p), ("w_scales", ctypes.c_void_p), ("w_format", ctypes.c_int),
+        ("x_codes", ctypes.c_void_p), ("x_scales", ctypes.c_void_p), ("x_format", ctypes.c_int),
+        ("offsets", ctypes.c_void_p),
+        ("d", ctypes.c_void_p),
+        ("rows", ctypes.c_int64), ("num_experts", ctypes.c_int64), ("N", ctypes.c_int64), ("K", ctypes.c_int64),
+    ]
+
+
+class MoeCombineArgs(ctypes.Structure):
+    _fields_ = [
+        ("y", ctypes.c_void_p), ("top_k_index", ctypes.c_void_p), ("top_k_weights", ctypes.c_void_p), ("weights_dtype", ctypes.c_int),
+        ("row_of_slot", ctypes.c_void_p),
+        ("tokens", ctypes.c_int64), ("top_k", ctypes.c_int), ("num_experts", ctypes.c_int), ("hidden", ctypes.c_int64),
+        ("out", ctypes.c_void_p),
+    ]
+
+
 _lib = None
 _lock = threading.Lock()
 
@@ -192,6 +221,9 @@ def lib() -> ctypes.CDLL:
         L.mxq_quantize_transposed.argtypes = [ctypes.POINTER(TransposedQuantArgs), i32, vp]
         L.mxq_rope_quantize_kv.restype = i32
         L.mxq_rope_quantize_kv.argtypes = [ctypes.POINTER(RopeQuantizeKVArgs), i32, vp]
+        for name, args in (("mxq_moe_route", MoeRouteArgs), ("mxq_moe_gemm", MoeGemmArgs), ("mxq_moe_combine", MoeCombineArgs)):
+            getattr(L, name).restype = i32
+            getattr(L, name).argtypes = [ctypes.POINTER(args), i32, vp]
         if L.mxq_version() != ABI_VERSION:
             raise RuntimeError(f"torchmx_b200: libmxq.so has ABI v{L.mxq_version()}, this package needs v{ABI_VERSION}: rebuild with `python -m torchmx_b200.build --force`")
         if L.mxq_arch() != 1000:

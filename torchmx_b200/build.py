@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "lib", "libmxq.so")
-SOURCES = ["mxq_api.cu", "mxq_quantize.cu", "mxq_dequantize.cu", "mxq_transcode.cu", "mxq_tmap.cu", "mxq_gemm.cu", "mxq_gemm_skinny.cu", "mxq_gemm_dequant.cu", "mxq_softmax.cu", "mxq_flash_attention.cu", "mxq_act_quant.cu", "mxq_glue.cu", "mxq_kv_cache.cu"]
+SOURCES = ["mxq_api.cu", "mxq_quantize.cu", "mxq_dequantize.cu", "mxq_transcode.cu", "mxq_tmap.cu", "mxq_gemm.cu", "mxq_gemm_skinny.cu", "mxq_gemm_dequant.cu", "mxq_softmax.cu", "mxq_flash_attention.cu", "mxq_act_quant.cu", "mxq_glue.cu", "mxq_kv_cache.cu", "mxq_moe.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

@@ -27,6 +27,9 @@ int launch_rope(const mxq_rope_args_t*, int, cudaStream_t, char*, size_t);
 int launch_heads_quantize(const void*, int64_t, int64_t, int64_t, int64_t, int, unsigned, void*, uint8_t*, cudaStream_t, char*, size_t);
 int launch_transposed_quantize(const mxq_transposed_quantize_args_t*, cudaStream_t, char*, size_t);
 int launch_rope_quantize_kv(const mxq_rope_quantize_kv_args_t*, cudaStream_t, char*, size_t);
+int launch_moe_route(const mxq_moe_route_args_t*, cudaStream_t, char*, size_t);
+int launch_moe_gemm(const mxq_moe_gemm_args_t*, int, cudaStream_t, char*, size_t);
+int launch_moe_combine(const mxq_moe_combine_args_t*, cudaStream_t, char*, size_t);
 }  // namespace mxq
 
 namespace {
@@ -88,7 +91,7 @@ int waves_override() { static int v = env_int("MXQ_WAVES"); return v > 0 ? v : 0
 extern "C" {
 
 const char* mxq_last_error(void) { return g_err; }
-int mxq_version(void) { return 5; }
+int mxq_version(void) { return 6; }
 int mxq_arch(void) { return 1000; }
 
 int mxq_quantize(const void* src, int src_dtype, int64_t n_blocks, int block_size, int elem, unsigned flags, void* codes, uint8_t* scales,
@@ -344,6 +347,89 @@ int mxq_rope_quantize_kv(const mxq_rope_quantize_kv_args_t* a, int device, void*
     char msg[400] = "";
     const int rc = mxq::launch_rope_quantize_kv(a, (cudaStream_t)stream, msg, sizeof(msg));
     return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_rope_quantize_kv: %s", msg);
+}
+
+// shared by the three mxq_moe_* entries: the routing table's extents
+static int moe_check_routing(const char* who, int64_t tokens, int top_k, int num_experts) {
+    if (top_k < 1 || top_k > MXQ_MOE_MAX_TOP_K) return fail(MXQ_ERR_INVALID, "%s: top_k %d outside 1..%d", who, top_k, MXQ_MOE_MAX_TOP_K);
+    if (num_experts < 1 || num_experts > MXQ_MOE_MAX_EXPERTS) return fail(MXQ_ERR_INVALID, "%s: num_experts %d outside 1..%d", who, num_experts, MXQ_MOE_MAX_EXPERTS);
+    if (tokens < 0 || tokens > MXQ_MOE_MAX_TOKENS) return fail(MXQ_ERR_INVALID, "%s: tokens %lld outside 0..%d", who, (long long)tokens, MXQ_MOE_MAX_TOKENS);
+    return MXQ_OK;
+}
+
+int mxq_moe_route(const mxq_moe_route_args_t* a, int device, void* stream) {
+    if (!a) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null args");
+    if (const int rc = moe_check_routing("mxq_moe_route", a->tokens, a->top_k, a->num_experts)) return rc;
+    if (!a->top_k_index) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null top_k_index");
+    if (!a->offsets) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null offsets");
+    if (!a->row_of_slot) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null row_of_slot");
+    if (!a->token_of_row) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null token_of_row");
+    const bool quant = a->codes || a->scales || a->x;
+    if (quant) {
+        if (!a->x) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null x (codes / scales given)");
+        if (!a->codes) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null codes (x given)");
+        if (!a->scales) return fail(MXQ_ERR_INVALID, "mxq_moe_route: null scales (x given)");
+        if (!valid_elem(a->elem)) return fail(MXQ_ERR_INVALID, "mxq_moe_route: unknown element type %d", a->elem);
+        if (a->hidden <= 0 || a->hidden % 32) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_route: hidden %lld is not a positive multiple of 32", (long long)a->hidden);
+        if (a->ldx < a->hidden || a->ldx % 8) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_route: ldx %lld must be >= hidden and a multiple of 8", (long long)a->ldx);
+        if ((uintptr_t)a->x % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_route: x is not 16-byte aligned");
+        if ((uintptr_t)a->codes % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_route: codes are not 16-byte aligned");
+    }
+    if (a->tokens == 0) return MXQ_OK;
+    DeviceScope scope(device);
+    if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_moe_route: selecting device");
+    char msg[400] = "";
+    const int rc = mxq::launch_moe_route(a, (cudaStream_t)stream, msg, sizeof(msg));
+    return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_moe_route: %s", msg);
+}
+
+int mxq_moe_gemm(const mxq_moe_gemm_args_t* a, int device, void* stream) {
+    if (!a) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null args");
+    if (a->num_experts < 1 || a->num_experts > MXQ_MOE_MAX_EXPERTS)
+        return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: num_experts %lld outside 1..%d", (long long)a->num_experts, MXQ_MOE_MAX_EXPERTS);
+    if (a->rows < 0 || a->N < 0 || a->K < 0) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: negative extent");
+    if (a->rows > (int64_t)MXQ_MOE_MAX_TOKENS * MXQ_MOE_MAX_TOP_K) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: rows %lld exceed %d", (long long)a->rows, MXQ_MOE_MAX_TOKENS * MXQ_MOE_MAX_TOP_K);
+    if (!a->w_codes) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null w_codes");
+    if (!a->w_scales) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null w_scales");
+    if (!a->x_codes) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null x_codes");
+    if (!a->x_scales) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null x_scales");
+    if (!a->offsets) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null offsets");
+    if (!a->d) return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: null d");
+    if (a->w_format < 0 || a->w_format > MXQ_OPERAND_E5M2_BYTES || a->x_format < 0 || a->x_format > MXQ_OPERAND_E5M2_BYTES)
+        return fail(MXQ_ERR_INVALID, "mxq_moe_gemm: unknown operand format %d / %d", a->w_format, a->x_format);
+    if (a->K == 0 || a->K % 128) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: K %lld is not a positive multiple of 128", (long long)a->K);
+    if (a->N == 0 || a->N % 128) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: N %lld is not a positive multiple of 128", (long long)a->N);
+    if ((uintptr_t)a->w_codes % 32) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: w_codes is not 32-byte aligned");
+    if ((uintptr_t)a->x_codes % 32) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: x_codes is not 32-byte aligned");
+    if ((uintptr_t)a->w_scales % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: w_scales is not 16-byte aligned");
+    if ((uintptr_t)a->x_scales % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: x_scales is not 16-byte aligned");
+    if ((uintptr_t)a->d % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_gemm: d is not 16-byte aligned");
+    if (a->rows == 0) return MXQ_OK;
+    DeviceScope scope(device);
+    if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_moe_gemm: selecting device");
+    char msg[400] = "";
+    const int rc = mxq::launch_moe_gemm(a, scope.cur, (cudaStream_t)stream, msg, sizeof(msg));
+    return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_moe_gemm: %s", msg);
+}
+
+int mxq_moe_combine(const mxq_moe_combine_args_t* a, int device, void* stream) {
+    if (!a) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null args");
+    if (const int rc = moe_check_routing("mxq_moe_combine", a->tokens, a->top_k, a->num_experts)) return rc;
+    if (a->weights_dtype != MXQ_HP_F32 && a->weights_dtype != MXQ_HP_BF16) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: weights_dtype %d", a->weights_dtype);
+    if (!a->y) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null y");
+    if (!a->top_k_index) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null top_k_index");
+    if (!a->top_k_weights) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null top_k_weights");
+    if (!a->row_of_slot) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null row_of_slot");
+    if (!a->out) return fail(MXQ_ERR_INVALID, "mxq_moe_combine: null out");
+    if (a->hidden <= 0 || a->hidden % 8) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_combine: hidden %lld is not a positive multiple of 8", (long long)a->hidden);
+    if ((uintptr_t)a->y % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_combine: y is not 16-byte aligned");
+    if ((uintptr_t)a->out % 16) return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_moe_combine: out is not 16-byte aligned");
+    if (a->tokens == 0) return MXQ_OK;
+    DeviceScope scope(device);
+    if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_moe_combine: selecting device");
+    char msg[400] = "";
+    const int rc = mxq::launch_moe_combine(a, (cudaStream_t)stream, msg, sizeof(msg));
+    return rc == MXQ_OK ? MXQ_OK : fail(rc, "mxq_moe_combine: %s", msg);
 }
 
 }  // extern "C"

@@ -38,6 +38,7 @@ def _swap_children(model: torch.nn.Module, replacement_fn: Callable, filter_fn: 
 def quantize_linear_(model: torch.nn.Module, qconfig: QLinearConfig, layer_filter: Optional[Callable[[str], bool]] = None) -> None:
     """Replace every module whose type is exactly `torch.nn.Linear` (lm_head included) with
     `MXInferenceLinear.from_float(mod, qconfig)`, in place (reference: quant_api.py:188-215).
+    Mixture-of-experts banks stored as 3-D parameters are not nn.Linear; `quantize_llm_` quantizes those.
 
     `layer_filter(fqn) -> bool` is a B200-side extension used by the layer-sharded multi-GPU
     driver: only layers whose qualified name passes the filter are quantized by this rank.
@@ -113,8 +114,11 @@ def _fuse_norms_(model: torch.nn.Module) -> None:
 def quantize_llm_(model: torch.nn.Module, qattention_config: QAttentionConfig, qmlp_config: QLinearConfig, fuse_rmsnorm: bool = False) -> None:
     """Quantize an LLM in place: every Llama / Qwen2 attention block becomes its MX version with `qattention_config`
     (projections as MXInferenceLinear; Q / K / V / attention-weights quantization when all four configs are given), every
-    MLP block its MX version with `qmlp_config`, and whatever nn.Linear is left (lm_head) an MXInferenceLinear with
-    `qmlp_config` (reference: quant_api.py:218-271)."""
+    MLP block its MX version with `qmlp_config`, every mixture-of-experts expert bank of transformers' Mixtral / Qwen2-MoE /
+    Qwen3-MoE / OLMoE models (3-D gate_up_proj / down_proj parameters) an `MXInferenceExperts` with `qmlp_config`, and whatever
+    nn.Linear is left (lm_head, shared experts) an MXInferenceLinear with `qmlp_config` (reference: quant_api.py:218-271; at the
+    transformers version the reference targets the experts were per-expert nn.Linear modules).  The routers stay as they are."""
+    from .layers.mx_experts import MXInferenceExperts, is_expert_bank
     from .layers.mx_llama_attention import ATTENTION_LAYERS, MLP_LAYERS
     logger.info("Quantizing the model by swapping the Attention and MLP layers")
     logger.info(f"Attention Layer Quantization config:\n{pformat(qattention_config)}\n")
@@ -128,6 +132,7 @@ def quantize_llm_(model: torch.nn.Module, qattention_config: QAttentionConfig, q
 
     with small_scale_arena():
         _swap_children(model, replacement_fn=replace, filter_fn=lambda mod, fqn: type(mod) in table)
+        _swap_children(model, replacement_fn=lambda mod: MXInferenceExperts.from_float(mod, qmlp_config), filter_fn=lambda mod, fqn: is_expert_bank(mod))
     quantize_linear_(model, qmlp_config)
     if fuse_rmsnorm:
         _fuse_norms_(model)
