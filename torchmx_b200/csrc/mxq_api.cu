@@ -8,8 +8,8 @@
 #include "mxq_common.cuh"
 
 namespace mxq {
-cudaError_t launch_quantize(const void*, int, int64_t, int, int, unsigned, void*, uint8_t*, int, int, int, cudaStream_t);
-cudaError_t launch_dequantize(const void*, const uint8_t*, int64_t, int, int, int, void*, int, int, int, cudaStream_t);
+cudaError_t launch_quantize(const void*, int, int64_t, int, int, unsigned, void*, uint8_t*, int, int64_t, int, int, cudaStream_t);
+cudaError_t launch_dequantize(const void*, const uint8_t*, int64_t, int, int, int, void*, int, int64_t, int, int, cudaStream_t);
 cudaError_t launch_dequantize_strided(const void*, const uint8_t*, int, const int64_t*, const int64_t*, const int64_t*, int, int, int, int,
                                       void*, cudaStream_t);
 cudaError_t launch_transcode(const void*, int, int64_t, void*, int, cudaStream_t);
@@ -72,6 +72,16 @@ int sm_count_of(int device) {
     return n;
 }
 
+// L2 bytes of `device`: K1 / K2 launches that stream more than this take their L2 evict-first, back-to-front variants
+int64_t l2_bytes_of(int device) {
+    static int cache[64];
+    if (device >= 0 && device < 64 && cache[device]) return cache[device];
+    int n = 0;
+    if (cudaDeviceGetAttribute(&n, cudaDevAttrL2CacheSize, device) != cudaSuccess || n <= 0) n = 126 << 20;
+    if (device >= 0 && device < 64) cache[device] = n;
+    return n;
+}
+
 bool valid_elem(int e) { return e >= MXQ_ELEM_E4M3 && e <= MXQ_ELEM_E5M2; }
 
 // developer knobs (not part of the reference-facing contract), read once:
@@ -106,7 +116,7 @@ int mxq_quantize(const void* src, int src_dtype, int64_t n_blocks, int block_siz
     DeviceScope scope(device);
     if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_quantize: selecting device");
     const cudaError_t e = mxq::launch_quantize(src, src_dtype, n_blocks, block_size, elem, flags, codes, scales, sm_count_of(scope.cur),
-                                               quant_ept_override(), waves_override(), (cudaStream_t)stream);
+                                               l2_bytes_of(scope.cur), quant_ept_override(), waves_override(), (cudaStream_t)stream);
     if (e == cudaErrorNotSupported && (flags & MXQ_FLAG_OPERAND_LAYOUT))
         return fail(MXQ_ERR_UNSUPPORTED_SHAPE, "mxq_quantize: MXQ_FLAG_OPERAND_LAYOUT needs a 4 / 6-bit element type, block 32, bf16 source and 32-byte aligned pointers");
     return e == cudaSuccess ? MXQ_OK : fail_cuda(e, "mxq_quantize: launch");
@@ -122,7 +132,8 @@ int mxq_dequantize(const void* codes, const uint8_t* scales, int64_t n_blocks, i
     if (elem == MXQ_ELEM_E2M1 && ((n_blocks * block_size) & 1)) return fail(MXQ_ERR_INVALID, "mxq_dequantize: float4_e2m1 needs an even element count");
     DeviceScope scope(device);
     if (scope.err != cudaSuccess) return fail_cuda(scope.err, "mxq_dequantize: selecting device");
-    const cudaError_t e = mxq::launch_dequantize(codes, scales, n_blocks, block_size, elem, dst_dtype, dst, sm_count_of(scope.cur), deq_cb_override(), waves_override(),
+    const cudaError_t e = mxq::launch_dequantize(codes, scales, n_blocks, block_size, elem, dst_dtype, dst, sm_count_of(scope.cur), l2_bytes_of(scope.cur),
+                                                 deq_cb_override(), waves_override(),
                                                  (cudaStream_t)stream);
     return e == cudaSuccess ? MXQ_OK : fail_cuda(e, "mxq_dequantize: launch");
 }

@@ -55,6 +55,45 @@ __device__ __forceinline__ void stg64_stream(void* p, uint2 r) {
     asm volatile("st.global.L1::no_allocate.v2.b32 [%0], {%1,%2};" ::"l"(p), "r"(r.x), "r"(r.y) : "memory");
 }
 
+// ---- the same accesses with an L2 evict-first policy (launches that stream more bytes than L2 holds) --------------------
+// A line touched this way is among the first L2 replaces, so the read-once streams of a large launch do not push out the lines
+// written at normal priority -- the codes a following dequantize reads back.  The policy is a per-instruction operand: no
+// device or stream state outlives the kernel.
+// Code bytes at the end of a large K1's output (and at the start of K2's back-to-front walk) that take the hints: 3/5 of L2.
+// Beyond them the codes cannot be in L2 and the hints only cost.  B200, 1000 W, bench.py's sweep: a window of 1 / 0.6 / 0.4 /
+// 0.25 L2 gave 1.170 / 1.166 / 1.171 / 1.183 ms per step (parent 1.208).
+inline int64_t l2_handoff_window(int64_t l2_bytes) { return l2_bytes * 3 / 5; }
+
+__device__ __forceinline__ uint64_t l2_evict_first_policy() {
+    uint64_t pol;
+    asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+    return pol;
+}
+__device__ __forceinline__ u32x8 ldg256_evict_first(const void* p, uint64_t pol) {
+    u32x8 r;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8], %9;"
+                 : "=r"(r.v[0]), "=r"(r.v[1]), "=r"(r.v[2]), "=r"(r.v[3]), "=r"(r.v[4]), "=r"(r.v[5]), "=r"(r.v[6]), "=r"(r.v[7])
+                 : "l"(p), "l"(pol));
+    return r;
+}
+__device__ __forceinline__ uint4 ldg128_evict_first(const void* p, uint64_t pol) {
+    uint4 r;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.b32 {%0,%1,%2,%3}, [%4], %5;"
+                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p), "l"(pol));
+    return r;
+}
+// one byte through the read-only path (what __ldg does), L1 allocating: the neighbouring lanes read the neighbouring bytes
+__device__ __forceinline__ uint32_t ldg8_evict_first(const uint8_t* p, uint64_t pol) {
+    uint32_t r;
+    asm volatile("ld.global.nc.L2::cache_hint.u8 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol));
+    return r;
+}
+__device__ __forceinline__ void stg256_evict_first(void* p, const u32x8& r, uint64_t pol) {
+    asm volatile("st.global.L1::no_allocate.L2::cache_hint.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8}, %9;" ::"l"(p), "r"(r.v[0]), "r"(r.v[1]),
+                 "r"(r.v[2]), "r"(r.v[3]), "r"(r.v[4]), "r"(r.v[5]), "r"(r.v[6]), "r"(r.v[7]), "l"(pol)
+                 : "memory");
+}
+
 // ---- E8M0 helpers -------------------------------------------------------------------------
 // shared exponent from the max of |bits| over the block (bf16: exponent field = bits >> 7)
 template <int ELEM>

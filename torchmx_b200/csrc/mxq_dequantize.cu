@@ -43,8 +43,8 @@ __device__ __forceinline__ void decode8_e2m1(uint32_t word, float sc, float (&f)
     }
 }
 
-template <int N, bool F32>
-__device__ __forceinline__ void store_run(void* dst, int64_t first_elem, const float (&f)[N]) {
+template <int N, bool F32, bool OVER_L2 = false>
+__device__ __forceinline__ void store_run(void* dst, int64_t first_elem, const float (&f)[N], uint64_t pol = 0) {
     // N consecutive outputs starting at element `first_elem`; N*sizeof(T) is a multiple of 32 and aligned
     if constexpr (F32) {
         uint8_t* p = reinterpret_cast<uint8_t*>(dst) + first_elem * 4;
@@ -62,59 +62,86 @@ __device__ __forceinline__ void store_run(void* dst, int64_t first_elem, const f
             u32x8 o;
 #pragma unroll
             for (int k = 0; k < 8; ++k) o.v[k] = pack_bf16x2(f[16 * j + 2 * k], f[16 * j + 2 * k + 1]);
-            stg256_stream(p + 32 * j, o);
+            if constexpr (OVER_L2) stg256_evict_first(p + 32 * j, o, pol);
+            else stg256_stream(p + 32 * j, o);
         }
     }
 }
 
-template <int ELEM, bool F32, int CB>
-__global__ void __launch_bounds__(kDequantThreads) dequantize_b32_kernel(const uint8_t* __restrict__ codes, const uint8_t* __restrict__ scales,
-                                                                         void* __restrict__ dst, int64_t n_code_bytes) {
+// One thread's chunk c of CB code bytes: decode with the block scales, store the values.
+template <int ELEM, bool F32, int CB, bool OVER_L2>
+__device__ __forceinline__ void dequantize_b32_chunk(const uint8_t* __restrict__ codes, const uint8_t* __restrict__ scales, void* __restrict__ dst,
+                                                     int64_t c, uint64_t pol) {
     // a thread owns CB = 16 or 32 consecutive code bytes; each 16-byte half is half a block (1-byte
     // codes) or a whole block (fp4) and carries its own scale byte
     constexpr int PER = (ELEM == MXQ_ELEM_E2M1) ? 2 : 1;  // elements per code byte
     constexpr int NH = CB / 16;
-    const int64_t n_chunks = n_code_bytes / CB;
-    const int64_t stride = (int64_t)gridDim.x * kDequantThreads;
-    for (int64_t c = (int64_t)blockIdx.x * kDequantThreads + threadIdx.x; c < n_chunks; c += stride) {
-        uint32_t w[CB / 4];
-        if constexpr (CB == 32) {
-            const u32x8 v = ldg256_stream(codes + c * 32);
+    uint32_t w[CB / 4];
+    if constexpr (CB == 32) {
+        const u32x8 v = OVER_L2 ? ldg256_evict_first(codes + c * 32, pol) : ldg256_stream(codes + c * 32);
 #pragma unroll
-            for (int k = 0; k < 8; ++k) w[k] = v.v[k];
-        } else {
-            const uint4 v = ldg128_stream(codes + c * 16);
-            w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
-        }
-        int s[NH];
+        for (int k = 0; k < 8; ++k) w[k] = v.v[k];
+    } else {
+        const uint4 v = OVER_L2 ? ldg128_evict_first(codes + c * 16, pol) : ldg128_stream(codes + c * 16);
+        w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
+    }
+    int s[NH];
 #pragma unroll
-        for (int h = 0; h < NH; ++h) s[h] = __ldg(scales + ((c * CB + 16 * h) * PER) / 32);
+    for (int h = 0; h < NH; ++h) {
+        const uint8_t* sp = scales + ((c * CB + 16 * h) * PER) / 32;
+        if constexpr (OVER_L2) s[h] = (int)ldg8_evict_first(sp, pol);
+        else s[h] = __ldg(sp);
+    }
 #pragma unroll
-        for (int h = 0; h < NH; ++h) {
-            const float sc = scale_f32(s[h]);
-            const int64_t e0 = (c * CB + 16 * h) * PER;
-            if constexpr (ELEM == MXQ_ELEM_E2M1) {
-                float f[32];
+    for (int h = 0; h < NH; ++h) {
+        const float sc = scale_f32(s[h]);
+        const int64_t e0 = (c * CB + 16 * h) * PER;
+        if constexpr (ELEM == MXQ_ELEM_E2M1) {
+            float f[32];
 #pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    float t[8];
-                    decode8_e2m1(w[4 * h + i], sc, t);
+            for (int i = 0; i < 4; ++i) {
+                float t[8];
+                decode8_e2m1(w[4 * h + i], sc, t);
 #pragma unroll
-                    for (int k = 0; k < 8; ++k) f[8 * i + k] = t[k];
-                }
-                store_run<32, F32>(dst, e0, f);
-            } else {
-                float f[16];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    float t[4];
-                    decode4<ELEM>(w[4 * h + i], sc, t);
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) f[4 * i + k] = t[k];
-                }
-                store_run<16, F32>(dst, e0, f);
+                for (int k = 0; k < 8; ++k) f[8 * i + k] = t[k];
             }
+            store_run<32, F32, OVER_L2>(dst, e0, f, pol);
+        } else {
+            float f[16];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                float t[4];
+                decode4<ELEM>(w[4 * h + i], sc, t);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) f[4 * i + k] = t[k];
+            }
+            store_run<16, F32, OVER_L2>(dst, e0, f, pol);
         }
+    }
+}
+
+// OVER_L2 (bf16 target, code + output bytes exceed L2): the CTAs walk the data back to front -- virtual CTA v
+// (v = blockIdx.x + k * gridDim.x) owns tile n_tiles - 1 - v, lanes ascending inside it -- so the first CTAs read the codes a
+// preceding K1 wrote last, which are still in L2.  In the first `hint_tiles` tiles (l2_handoff_window() bytes of codes) code, scale and
+// output accesses are evict-first, so consumed codes and the output are replaced before the codes still ahead of the walk;
+// past them there is nothing left in L2 to protect and the tiles stream as in the plain kernel.
+template <int ELEM, bool F32, int CB, bool OVER_L2 = false>
+__global__ void __launch_bounds__(kDequantThreads) dequantize_b32_kernel(const uint8_t* __restrict__ codes, const uint8_t* __restrict__ scales,
+                                                                         void* __restrict__ dst, int64_t n_code_bytes, int64_t hint_tiles = 0) {
+    const int64_t n_chunks = n_code_bytes / CB;
+    if constexpr (OVER_L2) {
+        const uint64_t pol = l2_evict_first_policy();
+        const int64_t n_tiles = (n_chunks + kDequantThreads - 1) / kDequantThreads;
+        for (int64_t v = blockIdx.x; v < n_tiles; v += gridDim.x) {
+            const int64_t c = (n_tiles - 1 - v) * kDequantThreads + threadIdx.x;
+            if (c >= n_chunks) continue;
+            if (v < hint_tiles) dequantize_b32_chunk<ELEM, F32, CB, true>(codes, scales, dst, c, pol);
+            else dequantize_b32_chunk<ELEM, F32, CB, false>(codes, scales, dst, c, 0);
+        }
+    } else {
+        const int64_t stride = (int64_t)gridDim.x * kDequantThreads;
+        for (int64_t c = (int64_t)blockIdx.x * kDequantThreads + threadIdx.x; c < n_chunks; c += stride)
+            dequantize_b32_chunk<ELEM, F32, CB, false>(codes, scales, dst, c, 0);
     }
 }
 
@@ -284,9 +311,24 @@ __global__ void __launch_bounds__(256) dequantize_transposed_b32_kernel(const ui
 }
 
 // ---- launchers -----------------------------------------------------------------------------------
+// The OVER_L2 variant for bf16 targets.  fp4 walks back to front without hints: its output is four times its code bytes and
+// the evict-first streams measured slower than the handoff saves (B200, 1000 W, 16384^2 after its K1: 104.5 -> 106.9 us with
+// all hints, 104.8 us without).  fp32 targets (output four / eight times the codes) keep the forward kernel.
+template <int ELEM, bool F32, int CB>
+static void launch_b32(int64_t l2_bytes, int grid, cudaStream_t stream, const uint8_t* codes, const uint8_t* scales, void* dst, int64_t n_code_bytes) {
+    if constexpr (!F32) {
+        if (n_code_bytes + n_code_bytes * (ELEM == MXQ_ELEM_E2M1 ? 4 : 2) > l2_bytes) {  // codes + bf16 output
+            const int64_t hint_tiles = ELEM == MXQ_ELEM_E2M1 ? 0 : l2_handoff_window(l2_bytes) / ((int64_t)kDequantThreads * CB);
+            dequantize_b32_kernel<ELEM, F32, CB, true><<<grid, kDequantThreads, 0, stream>>>(codes, scales, dst, n_code_bytes, hint_tiles);
+            return;
+        }
+    }
+    dequantize_b32_kernel<ELEM, F32, CB><<<grid, kDequantThreads, 0, stream>>>(codes, scales, dst, n_code_bytes);
+}
+
 template <int ELEM, bool F32>
-static cudaError_t launch_flat(const void* codes, const uint8_t* scales, int64_t n_blocks, int block_size, void* dst, int sm_count, int cb,
-                               int waves, cudaStream_t stream) {
+static cudaError_t launch_flat(const void* codes, const uint8_t* scales, int64_t n_blocks, int block_size, void* dst, int sm_count,
+                               int64_t l2_bytes, int cb, int waves, cudaStream_t stream) {
     if (n_blocks == 0) return cudaSuccess;
     if (block_size == 32 && ((uintptr_t)codes % 32) == 0 && ((uintptr_t)dst % 32) == 0) {
         const int64_t n_code_bytes = n_blocks * ((ELEM == MXQ_ELEM_E2M1) ? 16 : 32);
@@ -298,8 +340,8 @@ static cudaError_t launch_flat(const void* codes, const uint8_t* scales, int64_t
         const int64_t want = (n_chunks + kDequantThreads - 1) / kDequantThreads;
         const int64_t cap = waves > 0 ? (int64_t)sm_count * 8 * waves : (int64_t)0x7FFFFFFF;
         const int grid = (int)(want < cap ? want : cap);
-        if (cb == 32) dequantize_b32_kernel<ELEM, F32, 32><<<grid, kDequantThreads, 0, stream>>>((const uint8_t*)codes, scales, dst, n_code_bytes);
-        else dequantize_b32_kernel<ELEM, F32, 16><<<grid, kDequantThreads, 0, stream>>>((const uint8_t*)codes, scales, dst, n_code_bytes);
+        if (cb == 32) launch_b32<ELEM, F32, 32>(l2_bytes, grid, stream, (const uint8_t*)codes, scales, dst, n_code_bytes);
+        else launch_b32<ELEM, F32, 16>(l2_bytes, grid, stream, (const uint8_t*)codes, scales, dst, n_code_bytes);
         return cudaGetLastError();
     }
     // any other block size / alignment: the strided kernel on a 1-D view
@@ -367,9 +409,9 @@ static cudaError_t launch_strided(const void* codes, const uint8_t* scales, int 
     }
 
 cudaError_t launch_dequantize(const void* codes, const uint8_t* scales, int64_t n_blocks, int block_size, int elem, int dst_dtype, void* dst,
-                              int sm_count, int cb, int waves, cudaStream_t stream) {
+                              int sm_count, int64_t l2_bytes, int cb, int waves, cudaStream_t stream) {
     const bool f32 = dst_dtype == MXQ_HP_F32;
-#define CALL(E, F) launch_flat<E, F>(codes, scales, n_blocks, block_size, dst, sm_count, cb, waves, stream)
+#define CALL(E, F) launch_flat<E, F>(codes, scales, n_blocks, block_size, dst, sm_count, l2_bytes, cb, waves, stream)
     MXQ_DISPATCH_ELEM_DT(elem, f32, CALL)
 #undef CALL
 }

@@ -21,28 +21,36 @@ constexpr int kQuantThreads = 256;
 // OPERAND (fp4 / fp6, EPT 16 / 32): the codes leave in the packed tensor-core operand format (include/mxq.h MXQ_OPERAND_*_PACKED:
 // fp4 low nibble first, fp6 four codes in three bytes) instead of the reference layout -- what mxq_pack_operand would make of
 // them, without the extra launch and round trip; the codes themselves are the same.
-template <int ELEM, int EPT, int BS = 32, bool OPERAND = false>
+// OVER_L2 (block 32, reference layout; the launch's input + code bytes exceed L2): from chunk `hint_from` on -- the chunks
+// whose codes are the last l2_handoff_window() bytes the kernel writes -- the input is loaded L2 evict-first while codes and
+// scales are stored at normal priority, so the lines the kernel leaves in L2 are those codes, the ones K2, walking back to
+// front, reads first.  The chunks before stream as in the plain kernel: their codes cannot stay in L2 anyway.
+template <int ELEM, int EPT, int BS = 32, bool OPERAND = false, bool OVER_L2 = false>
 __global__ void __launch_bounds__(kQuantThreads) quantize_b32_bf16_kernel(const uint16_t* __restrict__ src, uint8_t* __restrict__ codes,
-                                                                           uint8_t* __restrict__ scales, int64_t n_blocks, uint32_t flags) {
+                                                                           uint8_t* __restrict__ scales, int64_t n_blocks, uint32_t flags,
+                                                                           int64_t hint_from = 0) {
     pdl_launch_dependents();       // a dependent MX GEMM may start streaming its weights while the activation is quantized
     constexpr int LPB = BS / EPT;  // lanes per MX block
     constexpr int NW = EPT / 2;    // 32-bit words of bf16 pairs per thread
     constexpr int NO = (ELEM == MXQ_ELEM_E2M1) ? NW / 4 : NW / 2;
+    uint64_t pol = 0;
+    if constexpr (OVER_L2) pol = l2_evict_first_policy();
     const int64_t n_chunks = n_blocks * LPB;
     const int64_t stride = (int64_t)gridDim.x * kQuantThreads;
     for (int64_t c0 = (int64_t)blockIdx.x * kQuantThreads; c0 < n_chunks; c0 += stride) {
         const int64_t c = c0 + threadIdx.x;
         const bool live = c < n_chunks;  // a block's LPB lanes are live together (n_chunks % LPB == 0)
+        const bool ef = OVER_L2 && c0 >= hint_from;  // uniform per CTA
         uint32_t w[NW];
         if (live) {
             const uint8_t* p = reinterpret_cast<const uint8_t*>(src) + c * (EPT * 2);
             if constexpr (EPT == 8) {
-                const uint4 v = ldg128_stream(p);
+                const uint4 v = ef ? ldg128_evict_first(p, pol) : ldg128_stream(p);
                 w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
             } else {
 #pragma unroll
                 for (int j = 0; j < NW / 8; ++j) {
-                    const u32x8 v = ldg256_stream(p + 32 * j);
+                    const u32x8 v = ef ? ldg256_evict_first(p + 32 * j, pol) : ldg256_stream(p + 32 * j);
 #pragma unroll
                     for (int k = 0; k < 8; ++k) w[8 * j + k] = v.v[k];
                 }
@@ -222,9 +230,22 @@ __global__ void codes_generic_kernel(const T* __restrict__ src, const uint8_t* _
 }
 
 // ---- launchers ---------------------------------------------------------------------------------
+template <int ELEM, int EPT>
+static void launch_b32_bf16(int64_t l2_bytes, int grid, cudaStream_t stream, const uint16_t* src, uint8_t* codes, uint8_t* scales, int64_t n_blocks,
+                            unsigned flags) {
+    constexpr int64_t kCodeBytes = (ELEM == MXQ_ELEM_E2M1) ? 16 : 32;  // per block
+    if (n_blocks * (64 + kCodeBytes) > l2_bytes) {                     // bf16 input + codes
+        const int64_t window = l2_handoff_window(l2_bytes) / kCodeBytes * (32 / EPT);  // chunks of the last window of codes
+        const int64_t hint_from = n_blocks * (32 / EPT) - window;
+        quantize_b32_bf16_kernel<ELEM, EPT, 32, false, true><<<grid, kQuantThreads, 0, stream>>>(src, codes, scales, n_blocks, flags, hint_from);
+    } else {
+        quantize_b32_bf16_kernel<ELEM, EPT><<<grid, kQuantThreads, 0, stream>>>(src, codes, scales, n_blocks, flags);
+    }
+}
+
 template <int ELEM>
 static cudaError_t launch_quantize_elem(const void* src, int src_dtype, int64_t n_blocks, int block_size, unsigned flags, void* codes,
-                                        uint8_t* scales, int sm_count, int ept_override, int waves, cudaStream_t stream) {
+                                        uint8_t* scales, int sm_count, int64_t l2_bytes, int ept_override, int waves, cudaStream_t stream) {
     if (n_blocks == 0) return cudaSuccess;
     const uintptr_t a_src = (uintptr_t)src, a_codes = (uintptr_t)codes;
     if (flags & MXQ_FLAG_OPERAND_LAYOUT) {
@@ -248,9 +269,9 @@ static cudaError_t launch_quantize_elem(const void* src, int src_dtype, int64_t 
         const int grid = (int)(want < cap ? want : cap);
         const uint16_t* s16 = (const uint16_t*)src;
         uint8_t* c8 = (uint8_t*)codes;
-        if (ept == 8) quantize_b32_bf16_kernel<ELEM, 8><<<grid, kQuantThreads, 0, stream>>>(s16, c8, scales, n_blocks, flags);
-        else if (ept == 32) quantize_b32_bf16_kernel<ELEM, 32><<<grid, kQuantThreads, 0, stream>>>(s16, c8, scales, n_blocks, flags);
-        else quantize_b32_bf16_kernel<ELEM, 16><<<grid, kQuantThreads, 0, stream>>>(s16, c8, scales, n_blocks, flags);
+        if (ept == 8) launch_b32_bf16<ELEM, 8>(l2_bytes, grid, stream, s16, c8, scales, n_blocks, flags);
+        else if (ept == 32) launch_b32_bf16<ELEM, 32>(l2_bytes, grid, stream, s16, c8, scales, n_blocks, flags);
+        else launch_b32_bf16<ELEM, 16>(l2_bytes, grid, stream, s16, c8, scales, n_blocks, flags);
         return cudaGetLastError();
     }
     if (src_dtype == MXQ_HP_BF16 && (a_src % 32) == 0 && (a_codes % 32) == 0 && (block_size == 8 || block_size == 16 || block_size == 64 || block_size == 128)) {
@@ -288,16 +309,18 @@ static cudaError_t launch_quantize_elem(const void* src, int src_dtype, int64_t 
 }
 
 cudaError_t launch_quantize(const void* src, int src_dtype, int64_t n_blocks, int block_size, int elem, unsigned flags, void* codes,
-                            uint8_t* scales, int sm_count, int ept_override, int waves, cudaStream_t stream) {
+                            uint8_t* scales, int sm_count, int64_t l2_bytes, int ept_override, int waves, cudaStream_t stream) {
+#define CALL(E) launch_quantize_elem<E>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, l2_bytes, ept_override, waves, stream)
     switch (elem) {
-    case MXQ_ELEM_E4M3: return launch_quantize_elem<MXQ_ELEM_E4M3>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
-    case MXQ_ELEM_E3M2: return launch_quantize_elem<MXQ_ELEM_E3M2>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
-    case MXQ_ELEM_E2M3: return launch_quantize_elem<MXQ_ELEM_E2M3>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
-    case MXQ_ELEM_E2M1: return launch_quantize_elem<MXQ_ELEM_E2M1>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
-    case MXQ_ELEM_INT8: return launch_quantize_elem<MXQ_ELEM_INT8>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
-    case MXQ_ELEM_E5M2: return launch_quantize_elem<MXQ_ELEM_E5M2>(src, src_dtype, n_blocks, block_size, flags, codes, scales, sm_count, ept_override, waves, stream);
+    case MXQ_ELEM_E4M3: return CALL(MXQ_ELEM_E4M3);
+    case MXQ_ELEM_E3M2: return CALL(MXQ_ELEM_E3M2);
+    case MXQ_ELEM_E2M3: return CALL(MXQ_ELEM_E2M3);
+    case MXQ_ELEM_E2M1: return CALL(MXQ_ELEM_E2M1);
+    case MXQ_ELEM_INT8: return CALL(MXQ_ELEM_INT8);
+    case MXQ_ELEM_E5M2: return CALL(MXQ_ELEM_E5M2);
     default: return cudaErrorInvalidValue;
     }
+#undef CALL
 }
 
 }  // namespace mxq
